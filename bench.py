@@ -2,6 +2,7 @@
 """Benchmark of record for the BALF inference hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--batch 64] [--nms windowed]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic input on every rank:
 uint8 images -> /255 + pad (D0) -> detector forward (D1-D3) -> border mask + NMS + top-2048
@@ -13,6 +14,8 @@ HBM; ``e2e`` = the same metric through the public host-buffer API (``demo_match.
 pinned host uint8 in, keypoint records back on the host, copies inside the timed region).
 ``--impl reference`` times the reference's CPU algorithm (the oracle restatement; the reference
 itself cannot travel to the GPU box) on the box's host cores.
+``--dump-outputs DIR`` writes what the timed path returned in its last step to DIR/<name>.npy (see dump_outputs):
+the inputs and weights are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -25,11 +28,13 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the tree as it found it (it may be read-only)
 
 import numpy as np
 import torch
 
 H, W, K_FEATURES = 480, 640, 2048
+DUMP_LIMIT_BYTES = 64 * 10 ** 6 - 4096  # 64 MB of --dump-outputs, less room for the four .npy headers
 METRIC = "images/sec detect+NMS+top-k @640x480"
 FLOP_PER_PADDED_PIXEL = 119496          # SURVEY.md 8d (Linear / matmul MACs x 2 only)
 
@@ -46,7 +51,11 @@ def parse():
     p.add_argument("--no-cpu-baseline", action="store_true")
     p.add_argument("--no-extras", action="store_true", help="development / profiling: only the configs[1] workload")
     p.add_argument("--chunk", type=int, default=0, help="development: images per internal detector pass (library default if 0)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
+    a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    return a
 
 
 def workload_name(a):
@@ -71,6 +80,23 @@ def model_cfg():
     from balf_b200.configs import config
     from balf_b200.utils import test_utils
     return test_utils.get_cfg_from_yaml_file(config.DEFAULT_CFG)["model"]
+
+
+def dump_outputs(path, xy, score, count):
+    """The keypoint records the timed path returns (every rank's after the all-gather), as float32 (coordinates and
+    counts are exact in it): xy.npy [N,K,2] (x, y), score.npy [N,K], count.npy [N]; rows beyond count are zero.
+    image.npy [N] holds the batch index of each row: all images, or, when they would exceed 64 MB, a fixed sample of them
+    (seed 0) that fits."""
+    per_image = 4 * (xy[0].numel() + score[0].numel() + 2)
+    n = len(count)
+    image = np.arange(n)
+    if n * per_image > DUMP_LIMIT_BYTES:
+        image = np.sort(np.random.default_rng(0).choice(n, DUMP_LIMIT_BYTES // per_image, replace=False))
+    rows = torch.from_numpy(image).to(xy.device)
+    os.makedirs(path, exist_ok=True)
+    for name, t in (("xy", xy), ("score", score), ("count", count)):
+        np.save(os.path.join(path, name + ".npy"), t.index_select(0, rows).cpu().numpy().astype(np.float32))
+    np.save(os.path.join(path, "image.npy"), image.astype(np.float32))
 
 
 # ------------------------------------------------------------------------------------------ clocks
@@ -522,6 +548,8 @@ def main():
     prof = capi.profile_report(reset=True)
     capi.profile_enable(False)
     clocks = sampler.stop() if sampler else None
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, *out)
 
     # end to end through the host-buffer API: every step's uint8 batch goes pinned host -> device and its keypoint
     # records come back device -> host inside the timed region.  DetectPipeline is the streaming form of

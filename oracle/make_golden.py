@@ -1,11 +1,12 @@
 """Generate ``tests/golden/*.npz`` by running the REFERENCE's own Python modules.
 
-TEST INFRASTRUCTURE.  Run in the build container only (needs /root/reference, which does not
-exist on the GPU box):   python -m oracle.make_golden
+TEST INFRASTRUCTURE.  Needs a checkout of the reference project at oracle/_ref (or at the path in
+BALF_REFERENCE):   python -m oracle.make_golden [r2]
 
-What is pinned by these vectors: detector forward (balf/model), HardNet
-(third_party/hardnet), and every NumPy helper of balf/utils/test_utils.py that the hot path
-touches.  The reference is run unmodified except for two shims, both recorded in the files:
+What is pinned by these vectors: the seed-0 state_dicts and the forward of the detector
+(balf/model) and of HardNet (third_party/hardnet), and every NumPy helper of
+balf/utils/test_utils.py that the hot path touches.  The reference is run unmodified except
+for two shims, both recorded in the files:
 
 * ``np.argsort`` is forced to ``kind='stable'`` while reference code runs, so that its four
   unstable sorts become deterministic (tie order = input order).  See oracle/postproc.py.
@@ -14,6 +15,7 @@ touches.  The reference is run unmodified except for two shims, both recorded in
   sub-pixel columns of the ``*_subpix`` arrays are NOT reference-pinned (key
   ``unpinned_subpixel`` = 1 in the file).
 """
+import hashlib
 import os
 import sys
 import types
@@ -23,7 +25,7 @@ import numpy as np
 import torch
 import yaml
 
-REF = "/root/reference"
+REF = os.environ.get("BALF_REFERENCE") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
 
 
@@ -78,6 +80,23 @@ def weight_digest(sd):
     s = sum(float(v.double().sum()) for v in sd.values())
     q = sum(float((v.double() ** 2).sum()) for v in sd.values())
     return np.array([s, q, float(len(sd))])
+
+
+def state_dict_fingerprint(sd):
+    """key order, shape, dtype and SHA-256 of the bytes of every tensor of a state_dict: pins it bit for bit in a few KB
+    (the tensors themselves would take ~10 MB)."""
+    return {"keys": np.array(list(sd)),
+            "shapes": np.array([",".join(map(str, v.shape)) for v in sd.values()]),
+            "dtypes": np.array([str(v.dtype) for v in sd.values()]),
+            "sha256": np.array([hashlib.sha256(v.detach().cpu().contiguous().numpy().tobytes()).hexdigest()
+                                for v in sd.values()])}
+
+
+def save_score_planes(path, score):
+    """a float32 map as its four little-endian byte planes: planes compress where interleaved floats do not, which keeps
+    the 480x640 map under 1 MB (tests/conftest.py: load_score_480x640 rebuilds it bit for bit)."""
+    planes = np.ascontiguousarray(score, "<f4").view(np.uint8).reshape(-1, 4).T.copy()
+    np.savez_compressed(path, score_480x640_planes=planes)
 
 
 def synth_image_u8(h, w, seed, channels=1):
@@ -137,7 +156,8 @@ def main():
         pts = np.stack([xs, ys, rb[ys, xs]]).astype(np.float64)
         out, inds = tu.nms_fast(pts, 480, 640, 15)
         g["nms_fast_out"], g["nms_fast_inds"] = out, inds.astype(np.int64)
-    np.savez(os.path.join(OUT, "postproc_480x640.npz"), **g)
+    save_score_planes(os.path.join(OUT, "postproc_480x640_score.npz"), g.pop("score_480x640"))
+    np.savez_compressed(os.path.join(OUT, "postproc_480x640.npz"), **g)
 
     # ------------------------------------------------------------------ small synthetic maps: ties, plateaus, zeros, edge cases
     rng = np.random.default_rng(7)
@@ -190,13 +210,16 @@ def main():
         oh = hn(xh)
     np.savez(os.path.join(OUT, "hardnet.npz"), weight_digest=weight_digest(hn.state_dict()),
              first_weight=hn.state_dict()["features.0.weight"].numpy(), out=oh.numpy())
+    fingerprints = {"detector": state_dict_fingerprint(sd), "hardnet": state_dict_fingerprint(hn.state_dict())}
+    np.savez_compressed(os.path.join(OUT, "state_dict.npz"),
+                        **{m + "_" + k: v for m, fp in fingerprints.items() for k, v in fp.items()})
     print("golden vectors written to", OUT)
     for f in sorted(os.listdir(OUT)):
         print("  %-28s %8d bytes" % (f, os.path.getsize(os.path.join(OUT, f))))
 
 
 def ref_metric_modules():
-    """balf/benchmark_test/{repeatability_tools,geometry_tools}.py imported from /root/reference (they import
+    """balf/benchmark_test/{repeatability_tools,geometry_tools}.py imported from the reference (they import
     torchvision, which is present, and torchgeometry.core.warp_perspective, which is stubbed: unused by the functions run)."""
     import importlib.util
     tgm = sys.modules.get("torchgeometry") or types.ModuleType("torchgeometry")
@@ -296,7 +319,7 @@ def main_r2():
     xh = torch.rand(2048, 1, 32, 32, generator=torch.Generator().manual_seed(4321))
     with torch.inference_mode():
         oh = torch.cat([hn(xh[i:i + 256]) for i in range(0, 2048, 256)])
-    np.savez(os.path.join(OUT, "r2_hardnet2048.npz"), out=oh.numpy())
+    np.savez_compressed(os.path.join(OUT, "r2_hardnet2048.npz"), out=oh.numpy())
 
     rt, gt = ref_metric_modules()
     Hm, (hs, ws), src, dst, src_ms, dst_ms = metric_inputs()

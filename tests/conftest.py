@@ -9,7 +9,6 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-REFERENCE = "/root/reference"
 
 
 def pytest_configure(config):
@@ -34,6 +33,13 @@ def _built_library():
 
 def load_golden(name):
     return np.load(os.path.join(GOLDEN, name))
+
+
+def load_score_480x640():
+    """The reference's score map of a 480x640 image (tests/golden/postproc_480x640_score.npz), rebuilt bit for bit from
+    the four byte planes it is stored as (oracle/make_golden.py: save_score_planes)."""
+    planes = load_golden("postproc_480x640_score.npz")["score_480x640_planes"]
+    return np.ascontiguousarray(planes.T).view("<f4").reshape(480, 640)
 
 
 @pytest.fixture(scope="session")

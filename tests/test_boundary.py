@@ -1,12 +1,12 @@
 """Host-side contract of the drop-in boundary (CPU only: no compute calls)."""
 import os
-import sys
 
 import numpy as np
 import pytest
 import torch
 
-from conftest import REFERENCE
+from conftest import load_golden
+from oracle.make_golden import state_dict_fingerprint
 
 
 def test_library_exports_every_declared_symbol():
@@ -33,23 +33,17 @@ def test_state_dict_layout(detector, hardnet):
     assert sum(v.numel() for k, v in hs.items() if k.endswith("weight")) == 1334560
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference tree not mounted")
 def test_state_dict_identical_to_reference(model_cfg, detector, hardnet):
-    sys.path.insert(0, REFERENCE)
-    try:
-        from balf.model import get_model as ref_get_model
-        from third_party.hardnet.hardnet_pytorch import HardNet as RefHardNet
-        torch.manual_seed(0)
-        ref = ref_get_model.load_model(model_cfg).state_dict()
-        torch.manual_seed(0)
-        ref_h = RefHardNet().state_dict()
-    finally:
-        sys.path.remove(REFERENCE)
-    for mine, theirs in ((detector.state_dict(), ref), (hardnet.state_dict(), ref_h)):
-        assert list(mine.keys()) == list(theirs.keys())
-        for k in mine:
-            assert mine[k].shape == theirs[k].shape and torch.equal(mine[k], theirs[k]), k
-    detector.load_state_dict(ref)                                    # reference checkpoints load strictly
+    """Key order, shapes, dtypes and the bytes of every tensor of the seed-0 state_dicts against the reference's
+    (tests/golden/state_dict.npz), and a state_dict of the reference's layout loads strictly."""
+    from balf_b200.model import get_model
+    g = load_golden("state_dict.npz")
+    for name, sd in (("detector", detector.state_dict()), ("hardnet", hardnet.state_dict())):
+        for field, got in state_dict_fingerprint(sd).items():
+            np.testing.assert_array_equal(got, g[name + "_" + field], err_msg="%s %s" % (name, field))
+    ref = {k: torch.zeros([int(n) for n in shape.split(",") if n], dtype=getattr(torch, dtype.split(".")[1]))
+           for k, shape, dtype in zip(g["detector_keys"], g["detector_shapes"], g["detector_dtypes"])}
+    get_model.load_model(model_cfg).load_state_dict(ref)             # reference checkpoints load strictly
 
 
 def test_checkpoint_loader_contract(tmp_path, model_cfg):

@@ -3,7 +3,10 @@ F1 patch sampling (balf_b200/csrc/patches.cu), H1 HardNet (hardnet.cu), M1 SMNN 
 public demo_match.extract_features / extract_matches chain.
 
 Floating-point stages carry their tolerance here; match indices are bit-exact given the same
-distance matrix (tie rule: lower index first)."""
+distance matrix (tie rule: lower index first).  The modules run on CUDA copies of the session fixtures, which stay on
+the CPU for the tests that use them there."""
+import copy
+
 import numpy as np
 import pytest
 import torch
@@ -34,6 +37,10 @@ def capi():
 
 def hn_state(hardnet):
     return {k: v.detach().clone() for k, v in hardnet.state_dict().items()}
+
+
+def on_gpu(module):
+    return copy.deepcopy(module).to(dev())
 
 
 # ------------------------------------------------------------------------------------------ F1
@@ -84,7 +91,7 @@ def test_patches_batched_counts():
 def test_hardnet_golden(hardnet):
     g = load_golden("hardnet.npz")
     x = torch.rand(8, 1, 32, 32, generator=torch.Generator().manual_seed(4321))
-    hn = hardnet.to(dev())
+    hn = on_gpu(hardnet)
     with torch.inference_mode():
         got = hn(x.to(dev())).cpu().numpy()
     tol = DESC_ATOL if getattr(hn, "precision", "fp32") == "fp32" else DESC_ATOL_TC
@@ -96,7 +103,7 @@ def test_hardnet_reference_golden_2048(hardnet):
     """the reference's own HardNet output on 2048 seeded patches (two internal passes of the chunked reference loop)"""
     want = load_golden("r2_hardnet2048.npz")["out"]
     x = torch.rand(2048, 1, 32, 32, generator=torch.Generator().manual_seed(4321))
-    hn = hardnet.to(dev())
+    hn = on_gpu(hardnet)
     with torch.inference_mode():
         got = hn(x.to(dev())).cpu().numpy()
     tc = getattr(hn, "precision", "fp32") != "fp32"
@@ -112,24 +119,21 @@ def test_hardnet_matches_oracle(hardnet, n):
     g = torch.Generator().manual_seed(100 + n)
     x = torch.rand(n, 1, 32, 32, generator=g)
     x[0] = x[0] * 0.01 + 0.5                                                      # low-contrast patch (input_norm)
-    hn = hardnet.to(dev())
+    hn = on_gpu(hardnet)
     with torch.inference_mode():
         got = hn(x.to(dev())).cpu()
-        want = ohardnet.hardnet_forward(hn_state(hardnet.cpu()), x)
-    hardnet.to(dev())
+        want = ohardnet.hardnet_forward(hn_state(hardnet), x)
     tol = DESC_ATOL if getattr(hn, "precision", "fp32") == "fp32" else DESC_ATOL_TC
     np.testing.assert_allclose(got.numpy(), want.numpy(), atol=tol, rtol=0)
 
 
 def test_hardnet_rejects_cpu_and_training(hardnet):
+    hn = on_gpu(hardnet)
     with pytest.raises(RuntimeError):
-        hardnet.to(dev())(torch.zeros(2, 1, 32, 32))
-    hardnet.train()
-    try:
-        with pytest.raises(RuntimeError):
-            hardnet(torch.zeros(2, 1, 32, 32, device=dev()))
-    finally:
-        hardnet.eval()
+        hn(torch.zeros(2, 1, 32, 32))
+    hn.train()
+    with pytest.raises(RuntimeError):
+        hn(torch.zeros(2, 1, 32, 32, device=dev()))
 
 
 # ------------------------------------------------------------------------------------------ M1
@@ -181,7 +185,7 @@ def test_extract_features_and_matches(detector, detector_sd, hardnet):
     from balf_b200.configs import config
     from balf_b200.demo import demo_match
     args = config.default_test_args()
-    det, hn = detector.to(dev()), hardnet.to(dev())
+    det, hn = on_gpu(detector), on_gpu(hardnet)
     rgb1 = synth_u8(200, 264, 21)
     noise = np.random.default_rng(5).integers(-2, 3, rgb1.shape[:2])[..., None]
     rgb2 = np.clip(rgb1.astype(np.int64) + noise, 0, 255).astype(np.uint8)
@@ -189,8 +193,7 @@ def test_extract_features_and_matches(detector, detector_sd, hardnet):
     k1, d1 = demo_match.extract_features(args, rgb1, gray1, det, hn, dev())
     assert k1.shape[1] == 2 and d1.shape == (len(k1), 128)
     # oracle descriptors at the SAME keypoints (isolates F1 + H1 from detector tolerance)
-    hn_sd = hn_state(hardnet.cpu())
-    hardnet.to(dev())
+    hn_sd = hn_state(hardnet)
     want_d, _ = pipeline.describe(args, hn_sd, gray1, k1)
     tol = 1e-4 if getattr(hn, "precision", "fp32") == "fp32" else DESC_ATOL_TC
     np.testing.assert_allclose(d1, want_d, atol=tol, rtol=0)

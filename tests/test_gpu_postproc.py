@@ -4,7 +4,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import load_golden
+from conftest import load_golden, load_score_480x640
 from oracle import postproc, postproc_c
 
 pytestmark = pytest.mark.gpu
@@ -49,7 +49,7 @@ def oracle_greedy(score, border, thr, r, k, ps=0, fast=True):
 
 def test_windowed_golden_map():
     g = load_golden("postproc_480x640.npz")
-    score = g["score_480x640"]
+    score = load_score_480x640()
     for k in (2048, 500, 5000):
         want = postproc.windowed_detect(score, 15, 15, k)
         got = gpu_windowed(score, k, 15, 15)[0]
@@ -60,7 +60,7 @@ def test_windowed_golden_map():
 
 def test_greedy_golden_map():
     g = load_golden("postproc_480x640.npz")
-    score = g["score_480x640"]
+    score = load_score_480x640()
     for name, thr, r in (("greedy_thr001", 0.001, 15), ("greedy_thr015", 0.015, 15), ("greedy_thr001_r4", 0.001, 4)):
         got = gpu_greedy(score, 8192, 15, thr, r)[0]
         want = oracle_greedy(score, 15, thr, r, 8192)
@@ -74,8 +74,7 @@ def test_greedy_golden_map():
 
 
 def test_greedy_topk_binds():
-    g = load_golden("postproc_480x640.npz")
-    score = g["score_480x640"]
+    score = load_score_480x640()
     for k in (1, 100, 777):
         np.testing.assert_array_equal(gpu_greedy(score, k, 15, 0.001, 15)[0], oracle_greedy(score, 15, 0.001, 15, k))
     k = 300                                                       # r = 4 keeps thousands: radix-select path
@@ -83,8 +82,7 @@ def test_greedy_topk_binds():
 
 
 def test_subpixel():
-    g = load_golden("postproc_480x640.npz")
-    score = g["score_480x640"]
+    score = load_score_480x640()
     for thr, ps in ((0.001, 4), (0.015, 5), (0.001, 3)):
         got = gpu_greedy(score, 2048, 15, thr, 15, ps)[0]
         want = oracle_greedy(score, 15, thr, 15, 2048, ps)
@@ -292,8 +290,7 @@ def test_greedy_cells_vs_whole_image_kernel_and_oracle():
 
 
 def test_greedy_cells_batch_crop_and_subpixel():
-    g = load_golden("postproc_480x640.npz")
-    score = g["score_480x640"]
+    score = load_score_480x640()
     rng = np.random.default_rng(2)
     batch = np.stack([score, score[::-1].copy(), np.roll(score, 37, 1), rng.random((480, 640), dtype=np.float32) * 0.03])
     padded = np.zeros((4, 512, 704), np.float32)

@@ -4,7 +4,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import load_golden, synth_u8, weight_digest
+from conftest import load_golden, load_score_480x640, synth_u8, weight_digest
 from oracle import detector as odet
 from oracle import hardnet as ohn
 from oracle import pipeline, postproc, postproc_c
@@ -75,7 +75,7 @@ def _assert_same_points(mine, ref):
 @pytest.mark.parametrize("impl", ["numpy", "c"])
 def test_postproc_480x640_vs_reference(impl):
     g = load_golden("postproc_480x640.npz")
-    score = g["score_480x640"]
+    score = load_score_480x640()
     rb = postproc.remove_borders(score, 15)
     nms = postproc.apply_nms if impl == "numpy" else postproc_c.apply_nms
     np.testing.assert_array_equal(np.flatnonzero(nms(rb, 15)), g["apply_nms15_idx"])
@@ -99,7 +99,7 @@ def test_postproc_480x640_vs_reference(impl):
 
 def test_nms_fast_indices_vs_reference():
     g = load_golden("postproc_480x640.npz")
-    rb = postproc.remove_borders(g["score_480x640"], 15)
+    rb = postproc.remove_borders(load_score_480x640(), 15)
     ys, xs = np.nonzero(rb >= np.float32(0.001))
     keep = postproc.greedy_nms(xs, ys, rb[ys, xs].astype(np.float64), 480, 640, 15)
     np.testing.assert_array_equal(keep, g["nms_fast_inds"])
@@ -111,7 +111,7 @@ def test_subpixel_restatement_vs_shimmed_reference():
     """unpinned third-party step (torchgeometry): checks only the reference-side arithmetic
     (patch extraction, normalisation, log) around the restated soft-argmax."""
     g = load_golden("postproc_480x640.npz")
-    rb = postproc.remove_borders(g["score_480x640"], 15)
+    rb = postproc.remove_borders(load_score_480x640(), 15)
     for name, thr, ps in (("greedy_thr001_subpix4", 0.001, 4), ("greedy_thr015_subpix5", 0.015, 5)):
         mine = postproc.get_points_direct_from_score_map(rb, thr, 15, True, ps)
         canon = lambda p: p[np.lexsort((np.round(p[:, 0]), np.round(p[:, 1]), -p[:, 3]))]   # tie groups: see above
