@@ -578,7 +578,6 @@ static size_t ws_layout(const balf_detector_arch& a, int Bc, int Hp, int Wp, voi
 
 extern int g_tc_trace_sel;        // detector_tc.cu
 extern int g_match_impl;          // match.cu
-extern int g_tc_variant;          // detector_tc.cu
 extern int g_greedy_impl;         // nms.cu
 extern int g_greedy_rounds;       // nms.cu
 extern int g_nms_tma;             // nms.cu
@@ -672,12 +671,11 @@ static int run_pool(const Workspace& ws, int Bc, int h, int wd, float* out, cuda
 using namespace balf;
 
 extern "C" int balf_debug_set(int key, int value) {
-    BALF_REQUIRE(key >= 0 && key <= 7, "unknown debug key %d", key);
+    BALF_REQUIRE(key >= 0 && key <= 7 && key != 4, "unknown debug key %d", key);
     if (key == 7) { g_nms_tma = value ? 1 : 0; return 0; }
     if (key == 6) { g_greedy_rounds = value < 0 ? 0 : value > 64 ? 64 : value; return 0; }
     if (key == 5) { g_greedy_impl = value ? 1 : 0; return 0; }
     if (key == 3) { g_match_impl = value ? 1 : 0; return 0; }
-    if (key == 4) { g_tc_variant = value; return 0; }
     if (key == 0) g_tc_mask = value & 0x1F;
     else if (key == 2) g_tc_trace_sel = value;
     else { BALF_REQUIRE(value >= 0 && value <= 64, "chunk must be in [0, 64] (0 = automatic)"); g_chunk_images = value; }
@@ -780,26 +778,26 @@ extern "C" int balf_detector_forward(const balf_detector_arch* arch, const float
         const DownW* d = w.down;
         int tiles = 0;
         if (tcm & 1) {
-            if (int e = tc_run_level_dispatch(0, xb, true, d[0], a, tc_blob, Bc, Hp, Wp, ws.u, ws.v, ws.r, ws.q, ws.partial, st, px, 0)) return e;
+            if (int e = tc_run_level_dispatch(0, xb, d[0], a, tc_blob, Bc, Hp, Wp, ws.u, ws.v, ws.r, ws.q, ws.partial, st, px, 0)) return e;
             if (int e = run_se<32>(ws, d[0], Bc, Hp * Wp, Hp * Wp / 64, st)) return e;
         } else if (int e = run_level<3, 32, 128, 128>(xb, true, w.down[0], Bc, Hp, Wp, ws, st, &tiles)) return e;
         if (int e = run_pool<32>(ws, Bc, Hp, Wp, ws.pooled[0], st, (tcm & 1) ? 1 + px : 0, (tcm & 2) && !px)) return e;
         if (tcm & 2) {
-            if (int e = tc_run_level_dispatch(1, ws.pooled[0], false, d[1], a, tc_blob, Bc, Hp / 2, Wp / 2, ws.u, ws.v, ws.r, ws.q, ws.partial, st, px, 0)) return e;
+            if (int e = tc_run_level_dispatch(1, ws.pooled[0], d[1], a, tc_blob, Bc, Hp / 2, Wp / 2, ws.u, ws.v, ws.r, ws.q, ws.partial, st, px, 0)) return e;
             if (int e = run_se<64>(ws, d[1], Bc, Hp * Wp / 4, Hp * Wp / 256, st)) return e;
         } else if (int e = run_level<32, 64, 128, 128>(ws.pooled[0], false, w.down[1], Bc, Hp / 2, Wp / 2, ws, st, &tiles)) return e;
         if (int e = run_pool<64>(ws, Bc, Hp / 2, Wp / 2, ws.pooled[1], st, (tcm & 2) ? 1 + px : 0, (tcm & 4) && !px)) return e;
         if (tcm & 4) {
-            if (int e = tc_run_level_dispatch(2, ws.pooled[1], false, d[2], a, tc_blob, Bc, Hp / 4, Wp / 4, ws.u, ws.v, ws.r, ws.q, ws.partial, st, px, px == 0)) return e;
+            if (int e = tc_run_level_dispatch(2, ws.pooled[1], d[2], a, tc_blob, Bc, Hp / 4, Wp / 4, ws.u, ws.v, ws.r, ws.q, ws.partial, st, px, px == 0)) return e;
             if (int e = run_se<128>(ws, d[2], Bc, Hp * Wp / 16, Hp * Wp / 1024, st)) return e;
         } else if (int e = run_level<64, 128, 64, 64>(ws.pooled[1], false, w.down[2], Bc, Hp / 4, Wp / 4, ws, st, &tiles)) return e;
         if (int e = run_pool<128>(ws, Bc, Hp / 4, Wp / 4, ws.pooled[2], st, ((tcm & 4) && !px) ? 3 : 0, (tcm & 8) && !px)) return e;
         if (tcm & 8) {
-            if (int e = tc_run_level_dispatch(3, ws.pooled[2], false, d[3], a, tc_blob, Bc, hc, wc, ws.u, ws.v, ws.r, ws.q, ws.partial, st, px, px == 0 && (tcm & 16) != 0)) return e;
+            if (int e = tc_run_level_dispatch(3, ws.pooled[2], d[3], a, tc_blob, Bc, hc, wc, ws.u, ws.v, ws.r, ws.q, ws.partial, st, px, px == 0 && (tcm & 16) != 0)) return e;
             if (int e = run_se<256>(ws, d[3], Bc, hc * wc, hc * wc / 64, st)) return e;
         } else if (int e = run_level<128, 256, 64, 32>(ws.pooled[2], false, w.down[3], Bc, hc, wc, ws, st, &tiles)) return e;
         if (tcm & 16) {
-            if (int e = tc_run_head(ws.r, ws.q, ws.scale, d[3], w.head, a, tc_blob, Bc, hc, wc,
+            if (int e = tc_run_head(ws.r, ws.q, ws.scale, a, tc_blob, Bc, hc, wc,
                                     logits ? logits + (size_t)b0 * nl * hc * wc : nullptr, prob + (size_t)b0 * Hp * Wp, st, px, px == 0 && (tcm & 8) != 0)) return e;
             continue;
         }

@@ -81,9 +81,9 @@ inline size_t walk_packed(const balf_detector_arch& a, const float* base, DetW* 
 // tensor-core path, detector_tc.cu: px = 0 single-rounded fp16 / tf32 operands (precision 1), px = 1 split precision (precision 2)
 size_t tc_blob_floats(const balf_detector_arch& a);
 int tc_pack_weights(const balf_detector_arch& a, const DetW& w, float* blob, cudaStream_t st);
-int tc_run_level_dispatch(int level, const float* xin, bool nchw, const DownW& w, const balf_detector_arch& a, const float* blob,
+int tc_run_level_dispatch(int level, const float* xin, const DownW& w, const balf_detector_arch& a, const float* blob,
                           int Bc, int h, int wd, float* u, float* v, float* r, float* q, float* partial, cudaStream_t st, int px, int r16);
-int tc_run_head(const float* r, const float* q, const float* scale, const DownW& w, const HeadW& hw, const balf_detector_arch& a,
+int tc_run_head(const float* r, const float* q, const float* scale, const balf_detector_arch& a,
                 const float* blob, int Bc, int hc, int wc, float* logits, float* prob, cudaStream_t st, int px, int r16);
 
 }  // namespace balf

@@ -15,7 +15,7 @@
 // block branch: one 8x8 block; merge / head: 64 consecutive pixels).  Thread (row = tid % 128, part = tid / 128)
 // owns one part (1 / TPR) of the channels of pixel row `row`; TMEM lane == row, so GELU, gating and softmax are
 // thread-local and LayerNorm needs one (sum, sum of squares) exchange between the parts of a row through shared
-// memory.  Stage 1 runs one thread per row in five independent tile groups per CTA (BranchCfgT).
+// memory.  Stage 1 runs one thread per row in five independent tile groups per CTA (BranchCfg).
 //
 // What the epilogues do NOT do: biases ride in the GEMM (one extra K = 8 MMA whose A operand is a
 // constant [1 1 0 ...] column block and whose B rows hold the bias split into tf32 hi + lo parts), and
@@ -43,21 +43,8 @@
 namespace balf {
 using namespace umma;
 
-// development experiments (NVCC_FLAGS=-DBALF_EXP=mask; results are WRONG, the timings show what a piece costs):
-// 1 no GELU math, 2 no shared-memory operand stores, 4 no TMEM loads, 8 no global stores of the branch kernels,
-// 16 no MMA issue / completion wait in the branch kernels
-#ifndef BALF_EXP
-#define BALF_EXP 0
-#endif
-#ifndef BALF_MERGE32_CTAS
-#define BALF_MERGE32_CTAS 3
-#endif
-#ifndef BALF_MERGE_TPR
-#define BALF_MERGE_TPR 2      // threads per pixel row of the stage 3-4 merge kernels (4 = 16 epilogue warps per SM: measured no gain, 0.85 -> 0.88 ms at C = 128)
-#endif
-#ifndef BALF_RC16_MINC
-#define BALF_RC16_MINC 32     // conv1 / conv2 of the merge kernels run on fp16 operands for C > this
-#endif
+constexpr int kMerge32Ctas = 3;         // CTAs per SM of the single-rounded stage-1 merge kernel (MergeBulkCfg::min_ctas)
+constexpr int kRc16MinC = 32;           // conv1 / conv2 of the merge kernels run on fp16 operands for C > this
 constexpr int TM = 128;                 // pixel rows per tile
 constexpr int NT2 = 256;                // threads per CTA (two per row)
 constexpr int kMaxSlot = 4;              // ring slots: per kernel family (G::nslot), sized from the shared-memory budget
@@ -224,7 +211,7 @@ template <int CIN, int C, int PX = 0> struct MergeG {
     // conv1 / conv2 (A operands written by the epilogues) run on fp16 operands at every stage
     // and dense2 as well: u' / v' arrive as fp16 tiles (C <= 128) or are converted by the loader (C = 256)
     __host__ __device__ static constexpr bool h16(int gi) {
-        return gi == MG_PD2A || gi == MG_PD2B || (gi == MG_CONV0 && CIN >= 8) || ((gi == MG_RC1 || gi == MG_RC2) && (PX || C > BALF_RC16_MINC));
+        return gi == MG_PD2A || gi == MG_PD2B || (gi == MG_CONV0 && CIN >= 8) || ((gi == MG_RC1 || gi == MG_RC2) && (PX || C > kRc16MinC));
     }
 };
 template <int C, int PX = 0> struct HeadG {
@@ -389,7 +376,6 @@ __device__ __forceinline__ unsigned long long mul2(unsigned long long a, unsigne
 // two GELUs: the polynomial is evaluated in t = -a (alternating coefficient signs) so that the last step is one FFMA2
 // relu(v) + t * e.  12 instructions per pair (4 FMNMX, 6 FFMA2, 2 MUFU) instead of 20.
 __device__ __forceinline__ void gelu_erf2(float& v0, float& v1) {
-    if (BALF_EXP & 1) return;
     const float t0 = fmaxf(-fabsf(v0), -5.6568542494923806f), t1 = fmaxf(-fabsf(v1), -5.6568542494923806f);
     const unsigned long long t = pk2(t0, t1);
     // degree-5 fit (scripts/fit_gelu.py): |err| < 3.7e-6 absolute, 20x below the tf32 rounding of the value it feeds;
@@ -427,11 +413,6 @@ __device__ __forceinline__ float lrelu02(float v) { return v > 0.0f ? v : 0.2f *
 // CH consecutive accumulator columns of this thread's row -> registers (tcgen05.ld is warp-collective)
 template <int CH>
 __device__ __forceinline__ void ld_row(uint32_t taddr, float (&v)[CH]) {
-    if (BALF_EXP & 4) {
-#pragma unroll
-        for (int i = 0; i < CH; ++i) v[i] = __uint_as_float(taddr + i) * 1e-30f;
-        return;
-    }
     if constexpr (CH == 16) {
         tmem_ld16(taddr, v);
     } else {
@@ -460,7 +441,6 @@ __device__ __forceinline__ void st_row(uint32_t taddr, const float (&v)[CH]) {
 // this thread's CH values -> A operand (chunk-major, 128 rows), columns [col0, col0 + CH), tf32-rounded
 template <int CH>
 __device__ __forceinline__ void row_to_a(const float (&v)[CH], float* region, int row, int col0) {
-    if (BALF_EXP & 2) { if (v[0] == 12345.678f) region[row] = v[1]; return; }
 #pragma unroll
     for (int j = 0; j < CH / 4; ++j)
         *reinterpret_cast<float4*>(region + ((size_t)(col0 / 4 + j) * TM + row) * 4) =
@@ -478,7 +458,6 @@ __device__ __forceinline__ void split_h2(float a, float b, uint32_t& hi, uint32_
 // LOC > 0 (split precision): the lo chunks follow LOC chunks (= K / 8) after the hi chunks
 template <int CH, int LOC = 0>
 __device__ __forceinline__ void row_to_a16(const float (&v)[CH], float* region, int row, int col0) {
-    if (BALF_EXP & 2) { if (v[0] == 12345.678f) region[row] = v[1]; return; }
 #pragma unroll
     for (int j = 0; j < CH / 8; ++j) {
         uint32_t h[4], l[4];
@@ -648,21 +627,10 @@ __device__ __forceinline__ void wait_done(uint64_t* done, uint32_t& phase) {
     fence_after_sync();
 }
 // same, and the issuing lane refills the (now entirely free) weight ring before joining the barrier
-// WW: every warp waits on the completion barrier itself (one polling lane per warp) -- no CTA / group barrier after the MMAs
-template <typename G, int NG = 1, int NTG = NT2, bool WW = false>
+template <typename G, int NG = 1, int NTG = NT2>
 __device__ __forceinline__ void wait_done_ring(uint64_t* done, uint32_t& phase, Ring& r, const TcPlan& p, bool w0, int grp = 0) {
-    if constexpr (WW) {
-        if (elect_one()) {
-            if (!(BALF_EXP & 16)) mbar_wait(done, phase & 1);
-            if (w0 && !G::resident) ring_top_up<G::nslot>(r, p);
-        }
-        __syncwarp();
-        ++phase;
-        fence_after_sync();
-        return;
-    }
     if (w0 && elect_one()) {
-        if (!(BALF_EXP & 16)) mbar_wait(done, phase & 1);
+        mbar_wait(done, phase & 1);
         if (!G::resident) ring_top_up<G::nslot>(r, p);
     }
     group_sync<NG, NTG>(grp);
@@ -967,42 +935,42 @@ __device__ __forceinline__ void conv0_row(const float4 x, const float* vec, int 
 }
 
 // ------------------------------------------------------------------------------------------ branch kernel
-// TPR = threads per pixel row (each owns C / TPR channels).  The default variant of a stage ("V0") is the round-1 layout
-// (two threads per row); variant 1 is one thread per row at C = 32 (half the per-row overhead instructions -- address
-// arithmetic, barriers, LayerNorm exchanges -- of a kernel that is bound by instruction issue) and four threads per row at
-// C >= 128 (16 epilogue warps instead of 8 on an SM whose epilogues are latency-bound).
-template <int C, int TPR_, int NG_, bool WW_ = false, int PX_ = 0> struct BranchCfgT {
-    static constexpr bool WW = WW_;                                // warps wait on the MMA completion barrier directly
-    static constexpr int PX = PX_;                                 // 1: split precision (fp16 hi + lo operands, see BranchG)
-    static constexpr int TPR = TPR_;
+// One configuration per stage.  TPR = threads per pixel row (each owns C / TPR channels), groups = tile groups per CTA:
+//   C = 32:       one thread per row, five tile groups: half the per-row overhead instructions (address arithmetic, barriers,
+//                 LayerNorm exchanges) of a kernel that is bound by instruction issue -- -30 % instructions, -13 % time
+//                 against two threads per row
+//   C = 64, 128:  two threads per row (two tile groups at C = 64); four threads per row measured no gain
+//   C = 256:      four threads per row: 16 epilogue warps instead of 8 on an SM whose epilogues are latency-bound, -10 %
+// PX = 1: split precision (fp16 hi + lo operands, see BranchG).
+template <int C, int PX> struct BranchCfg {
+    static constexpr int TPR = C == 32 ? 1 : C == 256 ? 4 : 2;
+    static constexpr int groups = C == 32 ? 5 : C == 64 ? 2 : 1;   // tile groups per CTA (shared resident weights)
     static constexpr int NTG = TM * TPR;                           // threads per tile group
     static constexpr int CH = C / TPR;
     // operand region of a group: the [128 x C] A operand (hi chunks, then lo chunks: PX); the token mixing reads the same layout
     static constexpr uint32_t region = (uint32_t)TM * C * (PX ? 4u : 2u);
     static constexpr bool park_u = C <= 128;                       // u stays in TMEM (else it round-trips through `out`)
-    static constexpr bool swz_out = false;                         // (round-1 layout: fp32 tiles in the swizzled panel layout)
     static constexpr bool h16_out = C <= 128;                      // u' / v' leave as fp16 tiles [C / 8 chunks][128 pixels][8 halves]: the operand
                                                                    // layout of the merge kernel's kind::f16 dense2, half the HBM bytes
     static constexpr int col_u = 0;
     static constexpr int col_y = park_u ? C : 0;
-    static constexpr int ncols = NG_ * tc_cols(col_y + 2 * C) > 512 ? col_y + 2 * C : tc_cols(col_y + 2 * C);   // TMEM columns per group
-    static constexpr int groups = NG_;                             // tile groups per CTA (shared resident weights)
+    static constexpr int ncols = groups * tc_cols(col_y + 2 * C) > 512 ? col_y + 2 * C : tc_cols(col_y + 2 * C);   // TMEM columns per group
     static constexpr uint32_t xch = TPR == 1 ? 0u : 2u * TPR * TM * 8u;   // LayerNorm exchange buffers per group
     static constexpr int SC = TPR == 1 ? 16 : TPR == 4 ? (CH < 32 ? CH : 32) : (CH > 64 ? 64 : CH);   // sub-chunks bound the live registers
 };
-template <int C, int PX = 0> struct BranchCfg : BranchCfgT<C, 2, (C <= 32 ? 4 : C <= 64 ? 2 : 1), false, PX> {};
 
-template <int CIN, int C, int BR, typename Cfg>
+template <int CIN, int C, int BR, int PX>
 __device__ __forceinline__ void tc_branch_body(const float* __restrict__ xin, const DownW& w, const TcPlan& plan, const UnitGeom& geo,
                                                float* __restrict__ out, float* __restrict__ scratch, unsigned char* smem) {
-    using G = BranchG<CIN, C, Cfg::PX>;
+    using Cfg = BranchCfg<C, PX>;
+    using G = BranchG<CIN, C, PX>;
     constexpr int CH = Cfg::CH, NG = Cfg::groups, TPR = Cfg::TPR, NTG = Cfg::NTG, SC = Cfg::SC;
-    constexpr bool X3 = Cfg::PX != 0;
+    constexpr bool X3 = PX != 0;
     constexpr int LOC = X3 ? C / 8 : 0;                                   // lo chunks of an A operand follow its C / 8 hi chunks
     constexpr bool XH = !X3 && CIN >= 8;                                  // the level input arrives as fp16 (pool_kernel, single-rounded path)
     // stage 4, single-rounded path: u' / v' leave as fp16 channels-last rows (the merge kernel's loaders take their 16-byte chunks as
     // operand chunks, like the pooled level inputs); the fp32 residual u then round-trips through `scratch`, not through `out`
-    constexpr bool CL16 = !Cfg::h16_out && !Cfg::swz_out && !X3;
+    constexpr bool CL16 = !Cfg::h16_out && !X3;
     float* const rt = CL16 ? scratch : out;
     constexpr int XM = XH ? 3 : X3 ? 2 : 1;
     static_assert(NG == 1 || G::resident, "tile groups share resident weights (no ring state per group)");
@@ -1095,9 +1063,9 @@ __device__ __forceinline__ void tc_branch_body(const float* __restrict__ xin, co
             }
             TC_TRACE(plan, it, 1);
             sync_for_mma<NG, NTG>(grp);
-            if (!(BALF_EXP & 16) && w0 && elect_one()) { issue_linear_t<G, BG_CONV0>(ring, plan, region_addr, ones_addr, tm + Cfg::col_y, true); commit(s.done); }
+            if (w0 && elect_one()) { issue_linear_t<G, BG_CONV0>(ring, plan, region_addr, ones_addr, tm + Cfg::col_y, true); commit(s.done); }
             TC_TRACE(plan, it, 2);
-            wait_done_ring<G, NG, NTG, Cfg::WW>(s.done, phase, ring, plan, w0, grp);
+            wait_done_ring<G, NG, NTG>(s.done, phase, ring, plan, w0, grp);
             TC_TRACE(plan, it, 3);
             ld_row<CH>(lane_base + Cfg::col_y + col0, v);
 #pragma unroll
@@ -1113,9 +1081,9 @@ __device__ __forceinline__ void tc_branch_body(const float* __restrict__ xin, co
         TC_TRACE(plan, it, 4);
         sync_for_mma<NG, NTG>(grp);
         // ---- this branch's half of dense1 -> GELU = u (residual, parked) -> LayerNorm (affine folded into gMLP dense1)
-        if (!(BALF_EXP & 16) && w0 && elect_one()) { issue_linear_t<G, BG_PD1>(ring, plan, region_addr, ones_addr, tm + Cfg::col_u, true); commit(s.done); }
+        if (w0 && elect_one()) { issue_linear_t<G, BG_PD1>(ring, plan, region_addr, ones_addr, tm + Cfg::col_u, true); commit(s.done); }
         TC_TRACE(plan, it, 5);
-        wait_done_ring<G, NG, NTG, Cfg::WW>(s.done, phase, ring, plan, w0, grp);
+        wait_done_ring<G, NG, NTG>(s.done, phase, ring, plan, w0, grp);
         TC_TRACE(plan, it, 6);
         {
             ld_row<CH>(lane_base + Cfg::col_u + col0, v);
@@ -1131,13 +1099,13 @@ __device__ __forceinline__ void tc_branch_body(const float* __restrict__ xin, co
         TC_TRACE(plan, it, 7);
         sync_for_mma<NG, NTG>(grp);
         // ---- gMLP dense1 (two halves) -> GELU; y1 parked, y2 -> LayerNorm -> [channel][token] operand
-        if (!(BALF_EXP & 16) && w0 && elect_one()) {
+        if (w0 && elect_one()) {
             issue_linear_t<G, BG_D1A>(ring, plan, region_addr, ones_addr, tm + Cfg::col_y, true);
             issue_linear_t<G, BG_D1B>(ring, plan, region_addr, ones_addr, tm + Cfg::col_y + C, true);
             commit(s.done);
         }
         TC_TRACE(plan, it, 8);
-        wait_done_ring<G, NG, NTG, Cfg::WW>(s.done, phase, ring, plan, w0, grp);
+        wait_done_ring<G, NG, NTG>(s.done, phase, ring, plan, w0, grp);
         TC_TRACE(plan, it, 9);
         {
             ld_row<CH>(lane_base + Cfg::col_y + col0, v);
@@ -1159,9 +1127,9 @@ __device__ __forceinline__ void tc_branch_body(const float* __restrict__ xin, co
         TC_TRACE(plan, it, 10);
         sync_for_mma<NG, NTG>(grp);
         // ---- token mixing, gating y1 * (y2' + 1)
-        if (!(BALF_EXP & 16) && w0 && elect_one()) { issue_mix_t<G, BG_WM, C>(ring, plan, region_addr, tm + Cfg::col_y + C); commit(s.done); }
+        if (w0 && elect_one()) { issue_mix_t<G, BG_WM, C>(ring, plan, region_addr, tm + Cfg::col_y + C); commit(s.done); }
         TC_TRACE(plan, it, 11);
-        wait_done_ring<G, NG, NTG, Cfg::WW>(s.done, phase, ring, plan, w0, grp);
+        wait_done_ring<G, NG, NTG>(s.done, phase, ring, plan, w0, grp);
         TC_TRACE(plan, it, 12);
         {
 #pragma unroll 1
@@ -1179,9 +1147,9 @@ __device__ __forceinline__ void tc_branch_body(const float* __restrict__ xin, co
         TC_TRACE(plan, it, 13);
         sync_for_mma<NG, NTG>(grp);
         // ---- dense2 + residual u -> out
-        if (!(BALF_EXP & 16) && w0 && elect_one()) { issue_linear_t<G, BG_D2>(ring, plan, region_addr, ones_addr, tm + Cfg::col_y, true); commit(s.done); }
+        if (w0 && elect_one()) { issue_linear_t<G, BG_D2>(ring, plan, region_addr, ones_addr, tm + Cfg::col_y, true); commit(s.done); }
         TC_TRACE(plan, it, 14);
-        wait_done_ring<G, NG, NTG, Cfg::WW>(s.done, phase, ring, plan, w0, grp);
+        wait_done_ring<G, NG, NTG>(s.done, phase, ring, plan, w0, grp);
         TC_TRACE(plan, it, 15);
         {
             // Full-sector stores: a lane's row chunks are 16 bytes, so a warp store of "chunk j of 32 rows" touches 32
@@ -1190,13 +1158,10 @@ __device__ __forceinline__ void tc_branch_body(const float* __restrict__ xin, co
             // sector of row 2i, then of row 2i+1 -- 16 full sectors per instruction.
             const bool odd = (threadIdx.x & 1) != 0;
             // (own_base counts elements of the tile format: halves of an fp16 tile -- twice as many per tile in split precision)
-            const size_t own_base = (Cfg::swz_out || Cfg::h16_out) ? ((size_t)img * npix + (pix & ~(TM - 1))) * C * (Cfg::h16_out && X3 ? 2 : 1)
-                                                                   : ((size_t)img * npix + pix) * C;
-            const int own_sw = pix & (TM - 1);
+            const size_t own_base = Cfg::h16_out ? ((size_t)img * npix + (pix & ~(TM - 1))) * C * (X3 ? 2 : 1)
+                                                 : ((size_t)img * npix + pix) * C;
             const size_t oth_base = __shfl_xor_sync(0xffffffffu, (unsigned long long)own_base, 1);
-            const int oth_sw = __shfl_xor_sync(0xffffffffu, own_sw, 1);
             const size_t base_a = odd ? oth_base : own_base, base_b = odd ? own_base : oth_base;   // rows 2i, 2i+1
-            const int sw_a = odd ? oth_sw : own_sw, sw_b = odd ? own_sw : oth_sw;
             if constexpr (CL16 && CH % 64 == 0) {
                 float hv[CH / 2];                                   // this thread's CH output channels as packed halves
 #pragma unroll
@@ -1235,7 +1200,7 @@ __device__ __forceinline__ void tc_branch_body(const float* __restrict__ xin, co
                     // tile; a lane stores 16 bytes per chunk -- neighbouring pixels (the other unit of the tile in the grid
                     // branch, the same block row in the block branch) complete the 32-byte sectors.  fp16 has the 11-bit
                     // significand of the tf32 operand this value would otherwise be rounded to; satfinite guards the range.
-                    __half* tile = reinterpret_cast<__half*>(out) + own_base + (size_t)own_sw * 8;
+                    __half* tile = reinterpret_cast<__half*>(out) + own_base + (size_t)(pix & (TM - 1)) * 8;
 #pragma unroll
                     for (int j = 0; j < SC / 8; ++j) {
                         uint32_t h[4], l[4];
@@ -1246,7 +1211,7 @@ __device__ __forceinline__ void tc_branch_body(const float* __restrict__ xin, co
                             if constexpr (X3) split_h2(lo, hi, h[e], l[e]);
                             else asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(h[e]) : "f"(hi), "f"(lo));
                         }
-                        if (valid && (!(BALF_EXP & 8) || h[0] == 0x12345678u)) {
+                        if (valid) {
                             *reinterpret_cast<uint4*>(tile + (size_t)((col0 + c) / 8 + j) * (TM * 8)) = make_uint4(h[0], h[1], h[2], h[3]);
                             if constexpr (X3)      // split precision: the tile is the merge kernel's [hi chunks | lo chunks] A operand
                                 *reinterpret_cast<uint4*>(tile + (size_t)(C / 8 + (col0 + c) / 8 + j) * (TM * 8)) = make_uint4(l[0], l[1], l[2], l[3]);
@@ -1273,9 +1238,9 @@ __device__ __forceinline__ void tc_branch_body(const float* __restrict__ xin, co
                     // u' / v' feed nothing but the merge GEMM: rounding them here (RN, as every operand) lets the merge
                     // kernel stream them into its operand regions asynchronously, no register pass.  Low bits cleared:
                     // the C >= 128 merge kernels round again when they load, which must be a no-op
-                    if ((BR == 1 || Cfg::swz_out) && !X3) o[j] = to_tf32_clean(o[j]);
+                    if (BR == 1 && !X3) o[j] = to_tf32_clean(o[j]);
                 }
-                if constexpr (SC % 32 == 0 && !X3 && !Cfg::swz_out) {      // full-line stores (see oct_store)
+                if constexpr (SC % 32 == 0 && !X3) {      // full-line stores (see oct_store)
                     oct_store<SC / 4>(out, ((size_t)img * npix + pix) * C + col0 + c, ostride, reinterpret_cast<const float*>(o), valid);
                     continue;
                 }
@@ -1287,14 +1252,9 @@ __device__ __forceinline__ void tc_branch_body(const float* __restrict__ xin, co
                     recv.z = __shfl_xor_sync(0xffffffffu, send.z, 1); recv.w = __shfl_xor_sync(0xffffffffu, send.w, 1);
                     const float4 to_a = odd ? recv : o[j], to_b = odd ? o[j + 1] : recv;     // (row 2i, row 2i+1), chunk j + odd
                     const int chunk = (col0 + c) / 4 + j + (odd ? 1 : 0);
-                    if (valid && (!(BALF_EXP & 8) || to_a.x == 12345.678f)) {        // both lanes of a pair belong to the same unit
-                        if (Cfg::swz_out) {
-                            *reinterpret_cast<float4*>(out + base_a + sw_off(sw_a, chunk)) = to_a;
-                            *reinterpret_cast<float4*>(out + base_b + sw_off(sw_b, chunk)) = to_b;
-                        } else {
-                            *reinterpret_cast<float4*>(out + base_a + 4 * chunk) = to_a;
-                            *reinterpret_cast<float4*>(out + base_b + 4 * chunk) = to_b;
-                        }
+                    if (valid) {        // both lanes of a pair belong to the same unit
+                        *reinterpret_cast<float4*>(out + base_a + 4 * chunk) = to_a;
+                        *reinterpret_cast<float4*>(out + base_b + 4 * chunk) = to_b;
                     }
                 }
             }
@@ -1304,19 +1264,11 @@ __device__ __forceinline__ void tc_branch_body(const float* __restrict__ xin, co
     tc_finish(*s.tmem_slot, tc_cols(Cfg::ncols * NG));
 }
 
-// V = 0: the round-1 layout; V = 1: see BranchCfgT
-template <int C, int V, int PX = 0> struct BranchSel { using Cfg = BranchCfg<C, PX>; };
-template <int PX> struct BranchSel<32, 1, PX> { using Cfg = BranchCfgT<32, 1, 5, false, PX>; };
-template <int PX> struct BranchSel<32, 2, PX> { using Cfg = BranchCfgT<32, 1, 5, true, PX>; };
-template <int PX> struct BranchSel<64, 1, PX> { using Cfg = BranchCfgT<64, 4, 2, false, PX>; };
-template <int PX> struct BranchSel<128, 1, PX> { using Cfg = BranchCfgT<128, 4, 1, false, PX>; };
-template <int PX> struct BranchSel<256, 1, PX> { using Cfg = BranchCfgT<256, 4, 1, false, PX>; };
-
-template <int CIN, int C, int BR, int V, int PX = 0>
-__global__ void __launch_bounds__(BranchSel<C, V, PX>::Cfg::NTG * BranchSel<C, V, PX>::Cfg::groups, 1)
+template <int CIN, int C, int BR, int PX>
+__global__ void __launch_bounds__(BranchCfg<C, PX>::NTG * BranchCfg<C, PX>::groups, 1)
 tc_branch_kernel(const float* __restrict__ xin, DownW w, TcPlan plan, UnitGeom geo, float* __restrict__ out, float* __restrict__ scratch) {
     extern __shared__ __align__(1024) unsigned char smem[];
-    tc_branch_body<CIN, C, BR, typename BranchSel<C, V, PX>::Cfg>(xin, w, plan, geo, out, scratch, smem);
+    tc_branch_body<CIN, C, BR, PX>(xin, w, plan, geo, out, scratch, smem);
 }
 
 
@@ -1352,9 +1304,9 @@ __device__ __forceinline__ void unit_channel_sums(const float* reg, int t, int t
 __device__ __forceinline__ int col0_of(int tid, int ch) { return (tid >> 7) * ch; }
 template <int C, int PX = 0> struct MergeCfg {
     // threads per pixel row.  scripts/tc_trace.py at C = 128: the two epilogues that also store q / r take 5.6 k + 7.1 k of a
-    // tile's 22 k cycles; four threads per row (16 warps) did not shorten them -- the 16-byte-per-row global stores touch 16
-    // different 128-byte lines per warp instruction and queue in the L1 (one line per cycle), not in the issue slots
-    static constexpr int TPR = (C >= 128 && PX == 0) ? BALF_MERGE_TPR : 2;
+    // tile's 22 k cycles; four threads per row (16 warps) did not shorten them (0.85 -> 0.88 ms) -- the 16-byte-per-row global
+    // stores touch 16 different 128-byte lines per warp instruction and queue in the L1 (one line per cycle), not in the issue slots
+    static constexpr int TPR = 2;
     static constexpr int NT = TM * TPR;
     static constexpr uint32_t xch = 2u * TPR * TM * 8u;
     static constexpr int CH = C / TPR;
@@ -1375,7 +1327,7 @@ template <int C, int PX = 0> struct MergeCfg {
 
 template <int CIN, int C, int PX = 0>
 __global__ void __launch_bounds__(MergeCfg<C, PX>::NT, MergeCfg<C, PX>::min_ctas)
-tc_merge_kernel(const float* __restrict__ xin, DownW w, TcPlan plan, UnitGeom geo, const float* __restrict__ uin,
+tc_merge_kernel(const float* __restrict__ xin, TcPlan plan, UnitGeom geo, const float* __restrict__ uin,
                 const float* __restrict__ vin, float* __restrict__ rout, float* __restrict__ qout, float* __restrict__ partial, int r16) {
     extern __shared__ __align__(1024) unsigned char smem[];
     using Cfg = MergeCfg<C, PX>;
@@ -1384,7 +1336,6 @@ tc_merge_kernel(const float* __restrict__ xin, DownW w, TcPlan plan, UnitGeom ge
     constexpr int HM = PX ? 2 : 1, LOC = PX ? C / 8 : 0;      // operand mode of the loaders, lo-chunk offset of a K = C operand
     constexpr bool XH = PX == 0 && CIN >= 8;                  // fp16 level input (pool_kernel, single-rounded path)
     constexpr int XM = XH ? 3 : HM;
-    (void)w;
     const TcShared s = carve(smem, Cfg::region, plan, 1, Cfg::xch);
     const int tid = threadIdx.x, row = tid & (TM - 1), half = tid >> 7;
     const int ntiles = (geo.total_units + 1) / 2;
@@ -1517,7 +1468,7 @@ tc_merge_kernel(const float* __restrict__ xin, DownW w, TcPlan plan, UnitGeom ge
             float rstd, shift;
             ld_row<CH>(lane_base + Cfg::col_acc + col0, v);
             float sum = 0.f, sq = 0.f;
-            constexpr int SC = TPR == 4 ? (CH < 32 ? CH : 32) : CH > 64 ? 64 : CH;
+            constexpr int SC = CH > 64 ? 64 : CH;
             unsigned long long s2 = pk2(0.f, 0.f), q2 = pk2(0.f, 0.f);
 #pragma unroll
             for (int c = 0; c < CH; c += SC) {
@@ -1632,7 +1583,7 @@ template <int CIN, int C, int PX = 0> struct MergeBulkCfg {
     static constexpr uint32_t xch = 2u * TM * 8u;                    // one LayerNorm exchange per tile: a single buffer
     static constexpr int col_acc = 0, col_x0 = C;
     static constexpr int ncols = tc_cols(cc0 ? C : 2 * C);
-    static constexpr int min_ctas = C <= 32 ? (PX ? 2 : BALF_MERGE32_CTAS) : 1;
+    static constexpr int min_ctas = C <= 32 ? (PX ? 2 : kMerge32Ctas) : 1;
 };
 
 template <int CIN, int C, int PX = 0>
@@ -2113,8 +2064,8 @@ static void tc_build_plans_px(const balf_detector_arch& a, const float* base, Tc
         tc_add(m, MG_CONV0, off, c, cin, !ebias, mcap, a.dims[l] >= 8 ? hm : 0);
         tc_add(m, MG_PD2A, off, c, c, false, mcap, hm);               // mirrors MergeG::h16
         tc_add(m, MG_PD2B, off, c, c, !ebias, mcap, hm);
-        tc_add(m, MG_RC1, off, c, c, !ebias, mcap, (px || c > BALF_RC16_MINC) ? hm : 0);
-        tc_add(m, MG_RC2, off, c, c, !ebias, mcap, (px || c > BALF_RC16_MINC) ? hm : 0);
+        tc_add(m, MG_RC1, off, c, c, !ebias, mcap, (px || c > kRc16MinC) ? hm : 0);
+        tc_add(m, MG_RC2, off, c, c, !ebias, mcap, (px || c > kRc16MinC) ? hm : 0);
         if (ebias) { m.ebias_off = (uint32_t)off; off += (size_t)4 * c * 4; }     // [conv.0, dense2, conv1, conv2][row][hi, lo, 0, 0]
     }
     TcPlan& h = P.head;
@@ -2239,51 +2190,31 @@ static int tc_launch_cfg(K kernel, size_t smem, int tmem_cols, int ntiles, int* 
 }
 
 
-#ifdef BALF_TC_MAIN
-int g_tc_variant = 0x41;     // debug hook (balf_debug_set key 4): per-stage branch-kernel variant, 2 bits per stage (BranchSel)
-#else
-extern int g_tc_variant;
-#endif
-
-template <int CIN, int C, int V, int PX>
+template <int CIN, int C, int PX>
 static int tc_launch_branches(const float* xin, const DownW& w, const TcPlans& P, int level, const UnitGeom& g, int ntiles,
                               float* u, float* v, float* su, float* sv, cudaStream_t st) {
-    using Cfg = typename BranchSel<C, V, PX>::Cfg;
+    using Cfg = BranchCfg<C, PX>;
     constexpr int NG = Cfg::groups;
     int grid = 0;
     for (int b = 0; b < 2; ++b) {
         const TcPlan& p = P.branch[level][b];
         const size_t smem = tc_smem_bytes(Cfg::region, p, NG, Cfg::xch);
         if (b == 0) {
-            if (int e = tc_launch_cfg(tc_branch_kernel<CIN, C, 0, V, PX>, smem, tc_cols(Cfg::ncols * NG), ntiles, &grid, NG, Cfg::NTG)) return e;
+            if (int e = tc_launch_cfg(tc_branch_kernel<CIN, C, 0, PX>, smem, tc_cols(Cfg::ncols * NG), ntiles, &grid, NG, Cfg::NTG)) return e;
             ProfScope ps(C == 32 ? "det_branch_grid_c32" : C == 64 ? "det_branch_grid_c64" : C == 128 ? "det_branch_grid_c128" : "det_branch_grid_c256", st);
-            tc_branch_kernel<CIN, C, 0, V, PX><<<grid, Cfg::NTG * NG, smem, st>>>(xin, w, p, g, u, su);
+            tc_branch_kernel<CIN, C, 0, PX><<<grid, Cfg::NTG * NG, smem, st>>>(xin, w, p, g, u, su);
         } else {
-            if (int e = tc_launch_cfg(tc_branch_kernel<CIN, C, 1, V, PX>, smem, tc_cols(Cfg::ncols * NG), ntiles, &grid, NG, Cfg::NTG)) return e;
+            if (int e = tc_launch_cfg(tc_branch_kernel<CIN, C, 1, PX>, smem, tc_cols(Cfg::ncols * NG), ntiles, &grid, NG, Cfg::NTG)) return e;
             ProfScope ps(C == 32 ? "det_branch_block_c32" : C == 64 ? "det_branch_block_c64" : C == 128 ? "det_branch_block_c128" : "det_branch_block_c256", st);
-            tc_branch_kernel<CIN, C, 1, V, PX><<<grid, Cfg::NTG * NG, smem, st>>>(xin, w, p, g, v, sv);
+            tc_branch_kernel<CIN, C, 1, PX><<<grid, Cfg::NTG * NG, smem, st>>>(xin, w, p, g, v, sv);
         }
     }
     return 0;
-}
-template <int CIN, int C, int PX>
-static int tc_run_branches(const float* xin, const DownW& w, const TcPlans& P, int level, const UnitGeom& g, int ntiles,
-                           float* u, float* v, float* su, float* sv, cudaStream_t st) {
-    const int var = (g_tc_variant >> (2 * level)) & 3;
-    if constexpr (C == 32) {
-        if (var == 1) return tc_launch_branches<CIN, C, 1, PX>(xin, w, P, level, g, ntiles, u, v, su, sv, st);
-        if (var == 2) return tc_launch_branches<CIN, C, 2, PX>(xin, w, P, level, g, ntiles, u, v, su, sv, st);
-    }
-    if constexpr (C == 64 || C == 128 || C == 256) {
-        if (var == 1) return tc_launch_branches<CIN, C, 1, PX>(xin, w, P, level, g, ntiles, u, v, su, sv, st);
-    }
-    return tc_launch_branches<CIN, C, 0, PX>(xin, w, P, level, g, ntiles, u, v, su, sv, st);
 }
 
 template <int CIN, int C, int PX>
 static int tc_run_level(const float* xin, const DownW& w, const TcPlans& P, int level, int Bc, int h, int wd,
                         float* u, float* v, float* r, float* q, float* partial, cudaStream_t st, int r16) {
-    (void)r16;
     UnitGeom g{h, wd, h / 8, wd / 8, h * wd / 64, Bc * (h * wd / 64), 1.0f / (float)(h * wd / 64), 1.0f / (float)(wd / 8), 1.0f / (float)(wd / 8)};
     BALF_REQUIRE(g.total_units < (1 << 23), "internal: %d units in one pass exceed the fast_div range", g.total_units);
     const int ntiles = (g.total_units + 1) / 2;
@@ -2291,7 +2222,7 @@ static int tc_run_level(const float* xin, const DownW& w, const TcPlans& P, int 
     BALF_REQUIRE((plan_matches<BranchG<CIN, C, PX>>(P.branch[level][0]) && plan_matches<BranchG<CIN, C, PX>>(P.branch[level][1]) &&
                   plan_matches<MergeG<CIN, C, PX>>(P.merge[level])), "internal: compile-time and packed GEMM plans differ (level %d)", level);
     // (r and q are free until the merge kernel writes them: scratch of the stage-4 branch kernels' residual round trip)
-    if (int e = tc_run_branches<CIN, C, PX>(xin, w, P, level, g, ntiles, u, v, r, q, st)) return e;
+    if (int e = tc_launch_branches<CIN, C, PX>(xin, w, P, level, g, ntiles, u, v, r, q, st)) return e;
     if constexpr (C <= 64) {
         const TcPlan& p = P.merge[level];
         BALF_REQUIRE(g.total_units % 2 == 0, "internal: odd unit count at stage %d", level);
@@ -2305,7 +2236,7 @@ static int tc_run_level(const float* xin, const DownW& w, const TcPlans& P, int 
         const size_t smem = tc_smem_bytes(MergeCfg<C, PX>::region, p, 1, MergeCfg<C, PX>::xch);
         if (int e = tc_launch_cfg(tc_merge_kernel<CIN, C, PX>, smem, MergeCfg<C, PX>::ncols, ntiles, &grid, 1, MergeCfg<C, PX>::NT)) return e;
         ProfScope ps(C == 128 ? "det_merge_c128" : "det_merge_c256", st);
-        tc_merge_kernel<CIN, C, PX><<<grid, MergeCfg<C, PX>::NT, smem, st>>>(xin, w, p, g, u, v, r, q, partial, r16);
+        tc_merge_kernel<CIN, C, PX><<<grid, MergeCfg<C, PX>::NT, smem, st>>>(xin, p, g, u, v, r, q, partial, r16);
     }
     BALF_COUNT_LAUNCH(3);
     BALF_LAUNCH_OK();
@@ -2352,16 +2283,14 @@ extern template int tc_level_px<1>(int, const float*, const DownW&, const balf_d
 extern template int tc_head_px<1>(const float*, const float*, const float*, const balf_detector_arch&, const float*, int, int, int, float*,
                                   float*, cudaStream_t, int);
 
-int tc_run_level_dispatch(int level, const float* xin, bool nchw, const DownW& w, const balf_detector_arch& a, const float* blob,
+int tc_run_level_dispatch(int level, const float* xin, const DownW& w, const balf_detector_arch& a, const float* blob,
                           int Bc, int h, int wd, float* u, float* v, float* r, float* q, float* partial, cudaStream_t st, int px, int r16) {
-    (void)nchw;
     return px ? tc_level_px<1>(level, xin, w, a, blob, Bc, h, wd, u, v, r, q, partial, st, r16)
               : tc_level_px<0>(level, xin, w, a, blob, Bc, h, wd, u, v, r, q, partial, st, r16);
 }
 
-int tc_run_head(const float* r, const float* q, const float* scale, const DownW& w, const HeadW& hw, const balf_detector_arch& a,
+int tc_run_head(const float* r, const float* q, const float* scale, const balf_detector_arch& a,
                 const float* blob, int Bc, int hc, int wc, float* logits, float* prob, cudaStream_t st, int px, int r16) {
-    (void)w; (void)hw;
     return px ? tc_head_px<1>(r, q, scale, a, blob, Bc, hc, wc, logits, prob, st, r16)
               : tc_head_px<0>(r, q, scale, a, blob, Bc, hc, wc, logits, prob, st, r16);
 }

@@ -1,6 +1,6 @@
 #!/bin/bash
 # Development helper: build/variants/<name>.so for each "name=NVCC_FLAGS" argument (separate object dirs), e.g.
-#   scripts/build_variants.sh base= nogelu=-DBALF_EXP=1
+#   scripts/build_variants.sh base= trace=-DBALF_TC_TRACE
 set -e
 for spec in "$@"; do
   name=${spec%%=*}; flags=${spec#*=}

@@ -18,6 +18,13 @@ def test_library_exports_every_declared_symbol():
     assert c.abi_version() == 1
 
 
+def test_debug_set_rejects_unknown_keys():
+    import balf_b200._capi as c
+    for key in (-1, 4, 8):
+        assert c.debug_set(key, 0) == -1, key
+        assert "unknown debug key %d" % key in c._last_error().decode()
+
+
 def test_state_dict_layout(detector, hardnet):
     sd = detector.state_dict()
     assert len(sd) == 167                                            # SURVEY.md appendix A
