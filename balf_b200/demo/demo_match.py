@@ -257,3 +257,38 @@ def extract_matches(args, im_rgb1, im_gray1, im_rgb2, im_gray2, detector, descri
     ids = _capi.match_smnn(torch.from_numpy(desc1).to(dev), torch.from_numpy(desc2).to(dev), 0.99)[1]
     ids = ids.cpu().numpy()
     return kpts1[ids[:, 0], :2], kpts2[ids[:, 1], :2]
+
+
+def find_homography_batch(pairs, ransac_thr=3.0, max_iters=2000, seed=0, device=None):
+    """RANSAC homographies of many match lists in one library call (semantics: include/balf_b200.h,
+    balf_find_homography_ransac).  pairs = [(pts1 [M_i,2], pts2 [M_i,2])] host arrays of any lengths -> [(H [3,3] float64 or
+    None, mask uint8 [M_i,1])], each entry in the return layout of ``cv2.findHomography(pts1, pts2, cv2.RANSAC, ransac_thr,
+    maxIters=max_iters)``.  H is None when the pair has fewer than 4 matches or no non-degenerate sample.  The lists go to
+    the device as one padded float64 buffer, and H and the masks come back in one copy."""
+    dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+    if not pairs:
+        return []
+    p = [(np.asarray(a, np.float64).reshape(-1, 2), np.asarray(b, np.float64).reshape(-1, 2)) for a, b in pairs]
+    for a, b in p:
+        if len(a) != len(b):
+            raise ValueError("find_homography: pts1 and pts2 have %d and %d rows" % (len(a), len(b)))
+    B, M = len(p), max(max(len(a) for a, _ in p), 1)
+    host = np.zeros(2 * B * M * 2 + B)                    # p1 [B,M,2], p2 [B,M,2], then the counts
+    pts = host[:4 * B * M].reshape(2, B, M, 2)
+    for i, (a, b) in enumerate(p):
+        pts[0, i, :len(a)], pts[1, i, :len(b)] = a, b
+    host[4 * B * M:] = [len(a) for a, _ in p]
+    buf = torch.from_numpy(host).to(dev)
+    d = buf[:4 * B * M].view(2, B, M, 2)
+    H, mask, _ = _capi.find_homography_ransac(d[0], d[1], buf[4 * B * M:].to(torch.int32), ransac_thr, max_iters, seed)
+    out = torch.cat([H.reshape(-1).view(torch.uint8), mask.reshape(-1)]).cpu().numpy()
+    Hs = out[:B * 72].view(np.float64).reshape(B, 3, 3)
+    masks = out[B * 72:].reshape(B, M)
+    return [(Hs[i].copy() if Hs[i, 2, 2] != 0 else None, masks[i, :len(a)].reshape(-1, 1).copy()) for i, (a, _) in enumerate(p)]
+
+
+def find_homography(pts1, pts2, ransac_thr=3.0, max_iters=2000, seed=0, device=None):
+    """GPU drop-in for ``cv2.findHomography(pts1, pts2, cv2.RANSAC, ransac_thr, maxIters=max_iters)`` on one match list
+    (e.g. the output of ``extract_matches``) -> (H [3,3] float64 or None, mask uint8 [M,1]).  The iteration count is fixed
+    (no confidence-driven early exit), so the result is a pure function of (points, ransac_thr, max_iters, seed)."""
+    return find_homography_batch([(pts1, pts2)], ransac_thr, max_iters, seed, device)[0]

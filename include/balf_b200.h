@@ -251,6 +251,37 @@ BALF_API int balf_resize_repeatability(const double* kp, int n1, const double* w
                                        void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Geometric verification of match lists: RANSAC homography, batched over image pairs.  No reference counterpart (the
+ * reference stops at the SMNN matches; its HPatches / GoPro evaluation parsers name the measure without implementing it):
+ * the semantics are defined here, restated in oracle/homography.py and checked against that restatement and against
+ * cv2.findHomography(RANSAC).  float64 throughout, no fused multiply-add, so a result is a pure function of
+ * (inputs, thr, iters, seed).
+ * p1, p2 float64 [B,M,2] = (x, y) of the matches of each pair, count int32 [B] valid rows per pair (clamped to [0, M]).
+ * Outputs: H float64 [B,9] (row-major, H[8] = 1) mapping p1 to p2, inlier_mask uint8 [B,M], n_inliers int32 [B].
+ *  - Sampling: hypothesis h (0 <= h < iters) of pair b draws its 4 indices from
+ *      stream = splitmix64(splitmix64(seed) ^ (b << 32 | h)),  index_c = splitmix64(stream + c) mod n,  c = 0, 1, ...
+ *    (splitmix64(z): z += 0x9E3779B97F4A7C15; z = (z ^ z >> 30) * 0xBF58476D1CE4E5B9; z = (z ^ z >> 27) *
+ *    0x94D049BB133111EB; z ^ z >> 31, all mod 2^64).  An index already in the sample is skipped; a hypothesis that has not
+ *    found 4 distinct indices after 32 counters is degenerate.
+ *  - Minimal solver: each image's 4 points are normalised to centroid 0 and mean distance sqrt(2) (sums in index order);
+ *    the 8x8 DLT system with h33 = 1 is solved by Gaussian elimination with partial pivoting (first maximum wins); then
+ *    H = T2^-1 Hn T1, scaled to H[8] = 1.  Degenerate (score -1): any 3 of the 4 points collinear in either image
+ *    (|cross product of two triangle edges| <= 1e-6 in normalised coordinates, or not a number), a pivot that is 0 or not
+ *    finite, or H[8] = 0 / not finite before the scaling.
+ *  - Inliers: w = (H p1)_z > 0 and |(H p1)_xy * (1 / w) - p2|^2 <= thr^2 (squared distances, no square root).
+ *    Score = inlier count; the winner of a pair is the highest score, the lowest h among equal scores.
+ *  - Refit: the winner's inliers are refitted with the same normalised DLT through its 8x8 normal equations and the same
+ *    elimination, the sums accumulated in a fixed order (oracle/homography.py restates it).  Each refit replaces H and its
+ *    inliers; the refits repeat while the inlier count grows, at most 8 times.  The outputs are the last H and its inliers.
+ *  - A pair with fewer than 4 matches or no non-degenerate hypothesis: H all zeros, n_inliers = 0, mask all zeros.
+ * Argument errors (< 0): thr <= 0 (or NaN), iters outside [1, 131072], M outside [0, 16384] (test_utils.K_MAX),
+ * B outside [0, 65535], a workspace smaller than balf_homography_workspace_bytes(B, M, iters). */
+BALF_API size_t balf_homography_workspace_bytes(int B, int M, int iters);
+BALF_API int balf_find_homography_ransac(const double* p1, const double* p2, const int32_t* count, int B, int M,
+                                         double thr, int iters, uint64_t seed, double* H, uint8_t* inlier_mask,
+                                         int32_t* n_inliers, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * SURVEY.md section 8(e): the one collective of the sharded path.  No reference counterpart (the reference is single-device,
  * demo/demo_match.py:29): image batches are partitioned over the ranks, every rank runs the whole pipeline on its shard, and
  * the fixed-size keypoint records are all-gathered over NCCL (NVLink 5 / NVSwitch).
