@@ -519,27 +519,43 @@ _homog_ransac = _sig("balf_find_homography_ransac", c_int, _P, _P, _P, c_int, c_
                      _P, _P, c_size_t, _P)
 
 
-def find_homography_ransac(p1, p2, count, thr, iters, seed):
-    """p1, p2 float64 [B,M,2] CUDA (x, y) of each pair's matches, count int32 [B] valid rows per pair -> (H float64 [B,3,3],
-    inlier mask uint8 [B,M], n_inliers int32 [B]) on the device; RANSAC semantics in include/balf_b200.h."""
+def _ransac(fn_ws, fn, name, p1, p2, count, thr, iters, seed):
     _need_cuda(p1, "the matched points")
     _need_cuda(p2, "the matched points")
     _need_cuda(count, "the match counts")
     a, b = p1.contiguous().double(), p2.contiguous().double()
     cnt = count.contiguous().to(torch.int32)
     if a.dim() != 3 or a.shape[2] != 2 or b.shape != a.shape or cnt.shape != (a.shape[0],):
-        raise ValueError("find_homography_ransac: p1, p2 must be [B,M,2] and count [B]")
+        raise ValueError("%s: p1, p2 must be [B,M,2] and count [B]" % name)
     B, M, _ = a.shape
     dev = a.device
-    H = torch.empty(B, 3, 3, dtype=torch.float64, device=dev)
+    out = torch.empty(B, 3, 3, dtype=torch.float64, device=dev)
     mask = torch.empty(B, M, dtype=torch.uint8, device=dev)
     n_in = torch.empty(B, dtype=torch.int32, device=dev)
-    nbytes = _homog_ws(B, M, int(iters))                 # 0 for arguments the call itself rejects
+    nbytes = fn_ws(B, M, int(iters))                     # 0 for arguments the call itself rejects
     ws = _workspace(dev, nbytes)
     with torch.cuda.device(dev):
-        _ok(_homog_ransac(_ptr(a), _ptr(b), _ptr(cnt), B, M, float(thr), int(iters), int(seed) & 0xFFFFFFFFFFFFFFFF, _ptr(H),
-                          _ptr(mask), _ptr(n_in), _ptr(ws), nbytes, _stream(dev)))
-    return H, mask, n_in
+        _ok(fn(_ptr(a), _ptr(b), _ptr(cnt), B, M, float(thr), int(iters), int(seed) & 0xFFFFFFFFFFFFFFFF, _ptr(out),
+               _ptr(mask), _ptr(n_in), _ptr(ws), nbytes, _stream(dev)))
+    return out, mask, n_in
+
+
+def find_homography_ransac(p1, p2, count, thr, iters, seed):
+    """p1, p2 float64 [B,M,2] CUDA (x, y) of each pair's matches, count int32 [B] valid rows per pair -> (H float64 [B,3,3],
+    inlier mask uint8 [B,M], n_inliers int32 [B]) on the device; RANSAC semantics in include/balf_b200.h."""
+    return _ransac(_homog_ws, _homog_ransac, "find_homography_ransac", p1, p2, count, thr, iters, seed)
+
+
+_fund_ws = _sig("balf_fundamental_workspace_bytes", c_size_t, c_int, c_int, c_int)
+_fund_ransac = _sig("balf_find_fundamental_ransac", c_int, _P, _P, _P, c_int, c_int, c_double, c_int, ctypes.c_uint64, _P, _P,
+                    _P, _P, c_size_t, _P)
+
+
+def find_fundamental_ransac(p1, p2, count, thr, iters, seed):
+    """p1, p2 float64 [B,M,2] CUDA (x, y) of each pair's matches, count int32 [B] valid rows per pair -> (F float64 [B,3,3]
+    with x2^T F x1 = 0, unit Frobenius norm, inlier mask uint8 [B,M], n_inliers int32 [B]) on the device; RANSAC semantics
+    in include/balf_b200.h (balf_find_fundamental_ransac)."""
+    return _ransac(_fund_ws, _fund_ransac, "find_fundamental_ransac", p1, p2, count, thr, iters, seed)
 
 
 _box_nms = _sig("balf_box_nms_map", c_int, _P, c_int, c_int, c_int, c_float, c_float, c_float, c_int, _P, _P, c_size_t, _P)

@@ -16,7 +16,7 @@ FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-std=c++17", "-O3", "-li
 
 
 # per-source flags: the float64 metric kernels follow the reference's unfused Python / NumPy arithmetic
-EXTRA = {"metrics.cu": ["-fmad=false"], "homography.cu": ["-fmad=false"]}
+EXTRA = {"metrics.cu": ["-fmad=false"], "homography.cu": ["-fmad=false"], "fundamental.cu": ["-fmad=false"]}
 
 
 def sources():

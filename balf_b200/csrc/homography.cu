@@ -17,75 +17,19 @@
 // Splitting the hypothesis from the scoring keeps the 8x9 elimination out of the scoring kernel.  With the solver inside,
 // the scoring kernel needs 106 registers and a 576-byte stack frame (2 CTAs of 256 threads per SM); split, it needs 60
 // registers and no stack (4 CTAs per SM).  DESIGN.md section 4.4 has the timing of both layouts.
-#include "common.cuh"
+#include "ransac.cuh"
 #include "../../include/balf_b200.h"
 
 namespace balf {
 namespace {
 
-typedef unsigned long long u64;
-
-constexpr int kMaxMatches = 16384;       // test_utils.K_MAX: the largest keypoint list the library produces
-constexpr int kMaxIters = 1 << 17;
 constexpr int kMaxDraws = 32;            // hash counters per hypothesis before the sample is declared degenerate
 constexpr int kRefitPasses = 8;          // least-squares refits of the winner, stopping early once the set stops growing
 constexpr double kCollinearTol = 1e-6;   // |cross| of two edges of a sample triangle, in normalised coordinates
-constexpr double kSqrt2 = 1.4142135623730951;
-constexpr int kScoreThreads = 256;
-constexpr int kHypThreads = 128;
-constexpr int kChunk = 1024;             // points per shared-memory chunk of the scoring kernel (32 KB)
-constexpr int kRefitThreads = 256;
 constexpr int kNormalTerms = 44;         // 36 upper-triangle entries of the 8x8 normal matrix + 8 right-hand sides
 
-__device__ __forceinline__ u64 splitmix64(u64 z) {
-    z += 0x9E3779B97F4A7C15ull;
-    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
-    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-    return z ^ (z >> 31);
-}
-
-// Gaussian elimination with partial pivoting on the augmented system a [8][9] -> h [8].  The pivot is the first row with
-// the largest |a[r][k]| (a NaN counts as the largest, like np.argmax); false when a pivot is 0 or not finite.  Loops are
-// unrolled so that the row swap is a set of selects on registers.
-__device__ __forceinline__ bool solve8(double (&a)[8][9], double (&h)[8]) {
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-        double best = fabs(a[k][k]);
-        int p = k;
-#pragma unroll
-        for (int r = k + 1; r < 8; ++r) {
-            const double v = fabs(a[r][k]);
-            if (!isnan(best) && (isnan(v) || v > best)) { best = v; p = r; }
-        }
-        if (!(best > 0.0 && best < __longlong_as_double(0x7ff0000000000000ll))) return false;
-#pragma unroll
-        for (int r = k + 1; r < 8; ++r)
-            if (p == r) {
-#pragma unroll
-                for (int c = k; c < 9; ++c) { const double t = a[k][c]; a[k][c] = a[r][c]; a[r][c] = t; }
-            }
-        const double d = a[k][k];
-#pragma unroll
-        for (int r = k + 1; r < 8; ++r) {
-            const double f = a[r][k] / d;
-#pragma unroll
-            for (int c = k + 1; c < 9; ++c) a[r][c] = a[r][c] - f * a[k][c];
-        }
-    }
-#pragma unroll
-    for (int k = 7; k >= 0; --k) {
-        double s = a[k][8];
-#pragma unroll
-        for (int c = k + 1; c < 8; ++c) s = s - a[k][c] * h[c];
-        h[k] = s / a[k][k];
-    }
-    return true;
-}
-
-// Normalisation (u, v) = ((x - cx) * s, (y - cy) * s) of each image.  The solved hn maps normalised points of image 1 to
-// those of image 2; H = T2^-1 Hn T1, scaled so that H[2][2] = 1.  False when H[2][2] is 0 or not finite.
-struct Norm { double cx1, cy1, s1, cx2, cy2, s2; };
-
+// The solved hn maps normalised points of image 1 to those of image 2 (Norm: ransac.cuh); H = T2^-1 Hn T1, scaled so that
+// H[2][2] = 1.  False when H[2][2] is 0 or not finite.
 __device__ __forceinline__ bool denormalise(const double (&hn)[8], const Norm& n, double (&H)[9]) {
     const double Hn[9] = {hn[0], hn[1], hn[2], hn[3], hn[4], hn[5], hn[6], hn[7], 1.0};
     double G[9];                                                     // Hn T1, T1 = [[s1, 0, -s1 cx1], [0, s1, -s1 cy1], [0, 0, 1]]
@@ -120,21 +64,19 @@ __device__ __forceinline__ bool is_inlier(const double (&H)[9], double x1, doubl
     return w > 0.0 && ((dx * dx) + (dy * dy)) <= thr2;
 }
 
+// The model of ransac_score_kernel / mark_inliers (ransac.cuh); H[8] = 0 marks a degenerate hypothesis.
+struct Homography {
+    static constexpr int kMinMatches = 4;
+    static __device__ __forceinline__ bool valid(const double (&H)[9]) { return H[8] != 0.0; }
+    static __device__ __forceinline__ bool inlier(const double (&H)[9], double x1, double y1, double x2, double y2,
+                                                  double thr2) {
+        return is_inlier(H, x1, y1, x2, y2, thr2);
+    }
+};
+
 __device__ __forceinline__ bool collinear3(double ax, double ay, double bx, double by, double cx, double cy) {
     const double dx1 = bx - ax, dy1 = by - ay, dx2 = cx - ax, dy2 = cy - ay;
     return !(fabs((dx1 * dy2) - (dy1 * dx2)) > kCollinearTol);       // NaN (coincident points) counts as collinear
-}
-
-// normalises 4 points in place -> centroid and scale
-__device__ __forceinline__ void normalise4(double (&x)[4], double (&y)[4], double& cx, double& cy, double& s) {
-    cx = (((x[0] + x[1]) + x[2]) + x[3]) / 4.0;
-    cy = (((y[0] + y[1]) + y[2]) + y[3]) / 4.0;
-    double d[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) { const double dx = x[i] - cx, dy = y[i] - cy; d[i] = sqrt((dx * dx) + (dy * dy)); }
-    s = kSqrt2 / ((((d[0] + d[1]) + d[2]) + d[3]) / 4.0);
-#pragma unroll
-    for (int i = 0; i < 4; ++i) { x[i] = (x[i] - cx) * s; y[i] = (y[i] - cy) * s; }
 }
 
 // DLT rows of one correspondence (u, v) -> (u', v') with h33 = 1:
@@ -144,32 +86,11 @@ __device__ __forceinline__ void dlt_rows(double u, double v, double up, double v
     b[0] = 0.0; b[1] = 0.0; b[2] = 0.0; b[3] = u; b[4] = v; b[5] = 1.0; b[6] = -(u * vp); b[7] = -(v * vp);
 }
 
-__device__ __forceinline__ int clamp_count(const int32_t* count, int b, int M) {
-    const int n = count[b];
-    return n < 0 ? 0 : (n > M ? M : n);
-}
-
 // hypothesis h of pair b (n valid matches) -> H; false for a degenerate sample
 __device__ __forceinline__ bool make_hypothesis(const double* __restrict__ p1, const double* __restrict__ p2, int n, int M, int b,
                                                 int h, u64 seed, double (&H)[9]) {
-    bool ok = n >= 4;
     int idx[4] = {0, 0, 0, 0};
-    if (ok) {
-        const u64 stream = splitmix64(splitmix64(seed) ^ (((u64)b << 32) | (u64)h));
-        int k = 0;
-        for (int c = 0; c < kMaxDraws && k < 4; ++c) {
-            const int i = (int)(splitmix64(stream + (u64)c) % (u64)n);
-            bool dup = false;
-#pragma unroll
-            for (int j = 0; j < 4; ++j) dup |= (j < k) && idx[j] == i;
-            if (!dup) {
-#pragma unroll
-                for (int j = 0; j < 4; ++j) if (j == k) idx[j] = i;
-                ++k;
-            }
-        }
-        ok = k == 4;
-    }
+    bool ok = n >= 4 && draw_sample<4, kMaxDraws>(seed, b, h, n, idx);
     if (ok) {
         const double* q1 = p1 + (size_t)b * M * 2;
         const double* q2 = p2 + (size_t)b * M * 2;
@@ -180,8 +101,8 @@ __device__ __forceinline__ bool make_hypothesis(const double* __restrict__ p1, c
             x2[j] = q2[2 * idx[j]]; y2[j] = q2[2 * idx[j] + 1];
         }
         Norm nm;
-        normalise4(x1, y1, nm.cx1, nm.cy1, nm.s1);
-        normalise4(x2, y2, nm.cx2, nm.cy2, nm.s2);
+        normalise<4>(x1, y1, nm.cx1, nm.cy1, nm.s1);
+        normalise<4>(x2, y2, nm.cx2, nm.cy2, nm.s2);
         const int tri[4][3] = {{0, 1, 2}, {0, 1, 3}, {0, 2, 3}, {1, 2, 3}};
 #pragma unroll
         for (int t = 0; t < 4; ++t) {
@@ -218,81 +139,8 @@ __global__ void __launch_bounds__(kHypThreads) ransac_hyp_kernel(const double* _
     for (int i = 0; i < 9; ++i) out[i] = ok ? H[i] : 0.0;
 }
 
-// key = (inliers + 1) << 32 | (0xFFFFFFFF - h): a degenerate hypothesis scores -1 (key < 2^32), the maximum key is the
-// highest count, and among equal counts the lowest hypothesis index.
-__global__ void __launch_bounds__(kScoreThreads) ransac_score_kernel(const double* __restrict__ p1, const double* __restrict__ p2,
-                                                                     const int32_t* __restrict__ count, int M, int iters,
-                                                                     double thr2, const double* __restrict__ hyp,
-                                                                     u64* __restrict__ best) {
-    __shared__ double4 pts[kChunk];
-    const int h = blockIdx.x * blockDim.x + threadIdx.x, b = blockIdx.y;
-    const int n = clamp_count(count, b, M);
-    if (n < 4) return;                                               // every hypothesis of the pair is degenerate
-    double H[9];
-    bool ok = h < iters;
-    if (ok) {
-        const double* src = hyp + ((size_t)b * iters + h) * 9;
-#pragma unroll
-        for (int i = 0; i < 9; ++i) H[i] = src[i];
-        ok = H[8] != 0.0;
-    }
-    const double* q1 = p1 + (size_t)b * M * 2;
-    const double* q2 = p2 + (size_t)b * M * 2;
-    int inl = 0;
-    for (int base = 0; base < n; base += kChunk) {
-        const int m = min(kChunk, n - base);
-        __syncthreads();
-        for (int i = threadIdx.x; i < m; i += blockDim.x) {
-            const size_t g = 2 * (size_t)(base + i);
-            pts[i] = make_double4(q1[g], q1[g + 1], q2[g], q2[g + 1]);
-        }
-        __syncthreads();
-        if (ok) {
-#pragma unroll 4
-            for (int i = 0; i < m; ++i) {
-                const double4 p = pts[i];
-                inl += is_inlier(H, p.x, p.y, p.z, p.w, thr2) ? 1 : 0;
-            }
-        }
-    }
-    u64 key = h < iters ? ((u64)(ok ? inl + 1 : 0) << 32) | (u64)(0xFFFFFFFFu - (unsigned)h) : 0ull;
-#pragma unroll
-    for (int o = 16; o; o >>= 1) {
-        const u64 v = __shfl_xor_sync(0xffffffffu, key, o);
-        key = v > key ? v : key;
-    }
-    if ((threadIdx.x & 31) == 0 && key) atomicMax(best + b, key);
-}
-
-// Block sum of K per-thread partials in a fixed order (restated by oracle/homography.py: block_sum): a tree inside each
-// warp (lane t += lane t + o, o = 16 .. 1), then a tree over the 8 warp sums (w += w + o, o = 4, 2, 1).
-template <int K>
-__device__ __forceinline__ void block_sum(double (&v)[K], double (*warp_part)[kRefitThreads / 32], double* out) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-    for (int q = 0; q < K; ++q) {
-        double s = v[q];
-#pragma unroll
-        for (int o = 16; o; o >>= 1) s = s + __shfl_down_sync(0xffffffffu, s, o);
-        if (lane == 0) warp_part[q][warp] = s;
-    }
-    __syncthreads();
-    for (int q = threadIdx.x; q < K; q += blockDim.x) {
-        double w[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) w[j] = warp_part[q][j];
-#pragma unroll
-        for (int o = 4; o; o >>= 1)
-#pragma unroll
-            for (int j = 0; j < o; ++j) w[j] = w[j] + w[j + o];
-        out[q] = w[0];
-    }
-    __syncthreads();
-}
-
-// One CTA per pair.  Thread t accumulates points t, t + 256, ... (a non-inlier adds 0.0) and block_sum combines them:
-//   pass A: sums of x1, y1, x2, y2 over the inliers -> centroids = sum / count;
-//   pass B: sums of the distances to the centroids -> s = sqrt(2) / (sum / count);
+// One CTA per pair.  refit_norm (ransac.cuh) normalises the inliers (passes A and B), then, with the same strided
+// per-thread sums and block_sum:
 //   pass C: the 36 upper-triangle entries a_i a_j + b_i b_j (row-major, i <= j) and the 8 right-hand sides a_i u' + b_i v'
 //           of the normal equations -> the same solve8 / denormalise as the minimal solver.
 // Each refit replaces the current H and its inliers (the least-squares fit is kept even when one more point fell inside
@@ -323,61 +171,11 @@ __global__ void __launch_bounds__(kRefitThreads) ransac_refit_kernel(const doubl
 #pragma unroll
     for (int i = 0; i < 9; ++i) H[i] = hyp[((size_t)b * iters + h) * 9 + i];
 
-    // inliers of G into mask -> count
-    auto mark = [&](const double (&G)[9]) {
-        if (t == 0) cnt_sh = 0;
-        __syncthreads();
-        int c = 0;
-        for (int i = t; i < n; i += blockDim.x) {
-            const bool in = is_inlier(G, q1[2 * i], q1[2 * i + 1], q2[2 * i], q2[2 * i + 1], thr2);
-            mask[i] = in ? 1 : 0;
-            c += in ? 1 : 0;
-        }
-#pragma unroll
-        for (int o = 16; o; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
-        if ((t & 31) == 0) atomicAdd(&cnt_sh, c);
-        __syncthreads();
-        const int r = cnt_sh;
-        __syncthreads();
-        return r;
-    };
-
-    int cnt = mark(H);
+    int cnt = mark_inliers<Homography>(H, q1, q2, n, thr2, mask, &cnt_sh);
     const int rows = (n + kRefitThreads - 1) / kRefitThreads;
     for (int pass = 0; pass < kRefitPasses && cnt >= 4; ++pass) {
         const uint8_t* m = mask;
-        const double dn = (double)cnt;
-        double sA[4] = {0.0, 0.0, 0.0, 0.0};
-        for (int r = 0; r < rows; ++r) {
-            const int i = r * kRefitThreads + t;
-            const bool in = i < n && m[i];
-            sA[0] = sA[0] + (in ? q1[2 * i] : 0.0);
-            sA[1] = sA[1] + (in ? q1[2 * i + 1] : 0.0);
-            sA[2] = sA[2] + (in ? q2[2 * i] : 0.0);
-            sA[3] = sA[3] + (in ? q2[2 * i + 1] : 0.0);
-        }
-        block_sum<4>(sA, warp_part, tot);
-        Norm nm;
-        nm.cx1 = tot[0] / dn; nm.cy1 = tot[1] / dn; nm.cx2 = tot[2] / dn; nm.cy2 = tot[3] / dn;
-        __syncthreads();
-        double sB[2] = {0.0, 0.0};
-        for (int r = 0; r < rows; ++r) {
-            const int i = r * kRefitThreads + t;
-            const bool in = i < n && m[i];
-            double d1 = 0.0, d2 = 0.0;
-            if (in) {
-                const double ax = q1[2 * i] - nm.cx1, ay = q1[2 * i + 1] - nm.cy1;
-                const double bx = q2[2 * i] - nm.cx2, by = q2[2 * i + 1] - nm.cy2;
-                d1 = sqrt((ax * ax) + (ay * ay));
-                d2 = sqrt((bx * bx) + (by * by));
-            }
-            sB[0] = sB[0] + d1;
-            sB[1] = sB[1] + d2;
-        }
-        block_sum<2>(sB, warp_part, tot);
-        nm.s1 = kSqrt2 / (tot[0] / dn);
-        nm.s2 = kSqrt2 / (tot[1] / dn);
-        __syncthreads();
+        const Norm nm = refit_norm(q1, q2, n, cnt, m, warp_part, tot);
         double sC[kNormalTerms];
 #pragma unroll
         for (int q = 0; q < kNormalTerms; ++q) sC[q] = 0.0;
@@ -412,7 +210,7 @@ __global__ void __launch_bounds__(kRefitThreads) ransac_refit_kernel(const doubl
         if (!ok_sh) break;
 #pragma unroll
         for (int i = 0; i < 9; ++i) H[i] = Hs[i];
-        const int c2 = mark(H);                                      // the sums above are complete: the mask is free
+        const int c2 = mark_inliers<Homography>(H, q1, q2, n, thr2, mask, &cnt_sh);                                      // the sums above are complete: the mask is free
         const bool grew = c2 > cnt;
         cnt = c2;
         if (!grew) break;
@@ -422,8 +220,6 @@ __global__ void __launch_bounds__(kRefitThreads) ransac_refit_kernel(const doubl
     for (int i = t; i < M; i += blockDim.x) mask_out[(size_t)b * M + i] = i < n ? mask[i] : 0;
 }
 
-size_t hyp_offset(int B) { return align_up((size_t)B * sizeof(u64), 256); }
-
 }  // namespace
 }  // namespace balf
 
@@ -431,7 +227,7 @@ using namespace balf;
 
 extern "C" size_t balf_homography_workspace_bytes(int B, int M, int iters) {
     if (B < 0 || M < 0 || iters < 1 || iters > kMaxIters) return 0;
-    return hyp_offset(B) + (size_t)B * iters * 9 * sizeof(double) + 256;
+    return best_bytes(B) + (size_t)B * iters * 9 * sizeof(double) + 256;
 }
 
 extern "C" int balf_find_homography_ransac(const double* p1, const double* p2, const int32_t* count, int B, int M, double thr,
@@ -450,7 +246,7 @@ extern "C" int balf_find_homography_ransac(const double* p1, const double* p2, c
     cudaStream_t st = (cudaStream_t)stream;
     unsigned char* base = reinterpret_cast<unsigned char*>(align_up((size_t)workspace, 256));
     u64* best = reinterpret_cast<u64*>(base);
-    double* hyp = reinterpret_cast<double*>(base + hyp_offset(B));
+    double* hyp = reinterpret_cast<double*>(base + best_bytes(B));
     const double thr2 = thr * thr;
     BALF_CUDA_OK(cudaMemsetAsync(best, 0, (size_t)B * sizeof(u64), st));
     {
@@ -459,7 +255,7 @@ extern "C" int balf_find_homography_ransac(const double* p1, const double* p2, c
     }
     {
         ProfScope p("ransac_score", st);
-        ransac_score_kernel<<<dim3(cdiv(iters, kScoreThreads), B), kScoreThreads, 0, st>>>(p1, p2, count, M, iters, thr2, hyp,
+        ransac_score_kernel<Homography><<<dim3(cdiv(iters, kScoreThreads), B), kScoreThreads, 0, st>>>(p1, p2, count, M, iters, thr2, hyp,
                                                                                            best);
     }
     {

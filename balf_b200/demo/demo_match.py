@@ -259,19 +259,17 @@ def extract_matches(args, im_rgb1, im_gray1, im_rgb2, im_gray2, detector, descri
     return kpts1[ids[:, 0], :2], kpts2[ids[:, 1], :2]
 
 
-def find_homography_batch(pairs, ransac_thr=3.0, max_iters=2000, seed=0, device=None):
-    """RANSAC homographies of many match lists in one library call (semantics: include/balf_b200.h,
-    balf_find_homography_ransac).  pairs = [(pts1 [M_i,2], pts2 [M_i,2])] host arrays of any lengths -> [(H [3,3] float64 or
-    None, mask uint8 [M_i,1])], each entry in the return layout of ``cv2.findHomography(pts1, pts2, cv2.RANSAC, ransac_thr,
-    maxIters=max_iters)``.  H is None when the pair has fewer than 4 matches or no non-degenerate sample.  The lists go to
-    the device as one padded float64 buffer, and H and the masks come back in one copy."""
+def _ransac_batch(estimate, name, pairs, ransac_thr, max_iters, seed, device):
+    """The padded batch of ``find_homography_batch`` / ``find_fundamental_batch``: the lists go to the device as one padded
+    float64 buffer, ``estimate`` (a ``_capi`` RANSAC call) runs once, and the 3x3 models and the masks come back in one
+    copy -> [(model [3,3] float64 or None, mask uint8 [M_i,1])]; None where the library returned all zeros (no model)."""
     dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
     if not pairs:
         return []
     p = [(np.asarray(a, np.float64).reshape(-1, 2), np.asarray(b, np.float64).reshape(-1, 2)) for a, b in pairs]
     for a, b in p:
         if len(a) != len(b):
-            raise ValueError("find_homography: pts1 and pts2 have %d and %d rows" % (len(a), len(b)))
+            raise ValueError("%s: pts1 and pts2 have %d and %d rows" % (name, len(a), len(b)))
     B, M = len(p), max(max(len(a) for a, _ in p), 1)
     host = np.zeros(2 * B * M * 2 + B)                    # p1 [B,M,2], p2 [B,M,2], then the counts
     pts = host[:4 * B * M].reshape(2, B, M, 2)
@@ -280,11 +278,20 @@ def find_homography_batch(pairs, ransac_thr=3.0, max_iters=2000, seed=0, device=
     host[4 * B * M:] = [len(a) for a, _ in p]
     buf = torch.from_numpy(host).to(dev)
     d = buf[:4 * B * M].view(2, B, M, 2)
-    H, mask, _ = _capi.find_homography_ransac(d[0], d[1], buf[4 * B * M:].to(torch.int32), ransac_thr, max_iters, seed)
-    out = torch.cat([H.reshape(-1).view(torch.uint8), mask.reshape(-1)]).cpu().numpy()
-    Hs = out[:B * 72].view(np.float64).reshape(B, 3, 3)
+    G, mask, _ = estimate(d[0], d[1], buf[4 * B * M:].to(torch.int32), ransac_thr, max_iters, seed)
+    out = torch.cat([G.reshape(-1).view(torch.uint8), mask.reshape(-1)]).cpu().numpy()
+    Gs = out[:B * 72].view(np.float64).reshape(B, 3, 3)
     masks = out[B * 72:].reshape(B, M)
-    return [(Hs[i].copy() if Hs[i, 2, 2] != 0 else None, masks[i, :len(a)].reshape(-1, 1).copy()) for i, (a, _) in enumerate(p)]
+    return [(Gs[i].copy() if Gs[i].any() else None, masks[i, :len(a)].reshape(-1, 1).copy()) for i, (a, _) in enumerate(p)]
+
+
+def find_homography_batch(pairs, ransac_thr=3.0, max_iters=2000, seed=0, device=None):
+    """RANSAC homographies of many match lists in one library call (semantics: include/balf_b200.h,
+    balf_find_homography_ransac).  pairs = [(pts1 [M_i,2], pts2 [M_i,2])] host arrays of any lengths -> [(H [3,3] float64 or
+    None, mask uint8 [M_i,1])], each entry in the return layout of ``cv2.findHomography(pts1, pts2, cv2.RANSAC, ransac_thr,
+    maxIters=max_iters)``.  H is None when the pair has fewer than 4 matches or no non-degenerate sample.  The lists go to
+    the device as one padded float64 buffer, and H and the masks come back in one copy."""
+    return _ransac_batch(_capi.find_homography_ransac, "find_homography", pairs, ransac_thr, max_iters, seed, device)
 
 
 def find_homography(pts1, pts2, ransac_thr=3.0, max_iters=2000, seed=0, device=None):
@@ -292,3 +299,25 @@ def find_homography(pts1, pts2, ransac_thr=3.0, max_iters=2000, seed=0, device=N
     (e.g. the output of ``extract_matches``) -> (H [3,3] float64 or None, mask uint8 [M,1]).  The iteration count is fixed
     (no confidence-driven early exit), so the result is a pure function of (points, ransac_thr, max_iters, seed)."""
     return find_homography_batch([(pts1, pts2)], ransac_thr, max_iters, seed, device)[0]
+
+
+def find_fundamental_batch(pairs, ransac_thr=3.0, max_iters=1000, seed=0, device=None):
+    """RANSAC fundamental matrices of many match lists in one library call (semantics: include/balf_b200.h,
+    balf_find_fundamental_ransac).  pairs = [(pts1 [M_i,2], pts2 [M_i,2])] host arrays of any lengths -> [(F [3,3] float64
+    or None, mask uint8 [M_i,1])], each entry in the return layout of ``cv2.findFundamentalMat(pts1, pts2, cv2.FM_RANSAC,
+    ransac_thr, maxIters=max_iters)``, with x2^T F x1 = 0.  F is None when the pair has fewer than 7 matches or no model."""
+    return _ransac_batch(_capi.find_fundamental_ransac, "find_fundamental", pairs, ransac_thr, max_iters, seed, device)
+
+
+def find_fundamental(pts1, pts2, ransac_thr=3.0, max_iters=1000, seed=0, device=None):
+    """GPU counterpart of ``cv2.findFundamentalMat(pts1, pts2, cv2.FM_RANSAC, ransac_thr, maxIters=max_iters)`` on one match
+    list (e.g. the output of ``extract_matches``) -> (F [3,3] float64 or None, mask uint8 [M,1]).  The differences from
+    cv2:
+    - F is scaled to unit Frobenius norm with its first largest-magnitude entry positive; cv2 divides by F[2,2] where it
+      can.  A fundamental matrix is defined up to scale only, so both describe the same epipolar geometry.
+    - The iteration count is fixed (no confidence-driven early exit), so the result is a pure function of (points,
+      ransac_thr, max_iters, seed).
+    - With exactly 7 matches cv2 returns all (up to 3) 7-point solutions stacked [9,3]; this runs RANSAC as usual and
+      returns the best single F.
+    Plane degeneracy is not handled: on a planar scene F fits the matches but the epipolar geometry is not determined."""
+    return find_fundamental_batch([(pts1, pts2)], ransac_thr, max_iters, seed, device)[0]

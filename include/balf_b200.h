@@ -282,6 +282,46 @@ BALF_API int balf_find_homography_ransac(const double* p1, const double* p2, con
                                          int32_t* n_inliers, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Geometric verification of match lists of general 3-D scenes: RANSAC fundamental matrix, batched over image pairs.  No
+ * reference counterpart (its GoPro evaluation parser, config_gopro_eval.py, names the measure without implementing it):
+ * the semantics are defined here, restated in oracle/fundamental.py and checked against that restatement and against
+ * cv2.findFundamentalMat.  float64, no fused multiply-add, and only + - * / sqrt and comparisons, so a result is a pure
+ * function of (inputs, thr, iters, seed).
+ * Inputs and outputs use the homography's layouts: p1, p2 float64 [B,M,2], count int32 [B] (clamped to [0, M]); outputs
+ * F float64 [B,9] (row-major) with x2^T F x1 = 0 (F maps p1 to epipolar lines in image 2), inlier_mask uint8 [B,M],
+ * n_inliers int32 [B].
+ *  - Sampling: the homography's hash streams unchanged (stream = splitmix64(splitmix64(seed) ^ (b << 32 | h)),
+ *    index_c = splitmix64(stream + c) mod n), drawing 7 distinct indices; a hypothesis that has not found them after 64
+ *    counters has no model.
+ *  - Minimal solver (7-point): each image's 7 points normalised to centroid 0 and mean distance sqrt(2) (sums in index
+ *    order); the 2-D null space {F1, F2} of the 7x9 system by the homography's partial-pivot elimination (F1: f8 = 1,
+ *    f7 = 0; F2: f8 = 0, f7 = 1; a pivot that is 0 or not finite: no model); the real roots lam of
+ *    det(lam F1 + (1 - lam) F2) = 0, a cubic whose roots are bracketed (its derivative's roots split the Cauchy bound
+ *    interval into monotone pieces) and bisected, so up to 3 models per hypothesis, model m of hypothesis h in slot
+ *    3 h + m; each model F = T2^T Fn T1.
+ *  - Scaling: every F has unit Frobenius norm and its first largest-magnitude entry positive (cv2 divides by F[8] where it
+ *    can; F is defined up to scale only).  A norm of 0 or not finite: no model.
+ *  - Inliers: with l2 = F x1 = (a, b, c), s = x2^T F x1 and l1 = F^T x2 = (a', b', c'), a match is an inlier when
+ *    s^2 <= thr^2 (a^2 + b^2) and s^2 <= thr^2 (a'^2 + b'^2), each a^2 + b^2 finite and > 0: both point-to-epipolar-line
+ *    distances are at most thr (cv2's FM_RANSAC error, squared).  The winner is the highest count, the lowest 3 h + m among
+ *    equal counts.
+ *  - Refit: when the winner has at least 8 inliers, the normalised 8-point least squares on them: the eigenvector of the
+ *    smallest eigenvalue of the 9x9 normal matrix (sums in the homography's fixed order) by cyclic Jacobi, made rank 2 in
+ *    normalised coordinates as F - (F v3) v3^T (v3 from a 3x3 Jacobi of F^T F: the nearest rank-2 matrix), denormalised
+ *    and scaled.  Each refit replaces F and its inliers; the refits repeat while the inlier count grows and is at least 8,
+ *    at most 8 times.
+ *  - A pair with fewer than 7 matches or no model: F all zeros, n_inliers = 0, mask all zeros.  With exactly 7 matches
+ *    cv2 returns all (up to 3) solutions stacked; this runs RANSAC as usual and returns the best one.
+ *  - Limits: plane degeneracy is not handled (no DEGENSAC).  On a planar scene (or a pure rotation) the returned F fits
+ *    the matches but the epipolar geometry is not determined by them.
+ * Argument errors (< 0): thr <= 0 (or NaN), iters outside [1, 131072], M outside [0, 16384], B outside [0, 65535], a
+ * workspace smaller than balf_fundamental_workspace_bytes(B, M, iters). */
+BALF_API size_t balf_fundamental_workspace_bytes(int B, int M, int iters);
+BALF_API int balf_find_fundamental_ransac(const double* p1, const double* p2, const int32_t* count, int B, int M,
+                                          double thr, int iters, uint64_t seed, double* F, uint8_t* inlier_mask,
+                                          int32_t* n_inliers, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * SURVEY.md section 8(e): the one collective of the sharded path.  No reference counterpart (the reference is single-device,
  * demo/demo_match.py:29): image batches are partitioned over the ranks, every rank runs the whole pipeline on its shard, and
  * the fixed-size keypoint records are all-gathered over NCCL (NVLink 5 / NVSwitch).
