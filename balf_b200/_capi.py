@@ -107,6 +107,13 @@ def _need_cuda(t, what):
         raise RuntimeError("balf_b200 has no CPU path: %s must be a CUDA tensor" % what)
 
 
+def _same_device(t, ref, what):
+    """t must be a CUDA tensor on ref's device: the C-ABI takes raw pointers and one stream."""
+    _need_cuda(t, what)
+    if t.device != ref.device:
+        raise ValueError("%s is on %s, expected %s" % (what, t.device, ref.device))
+
+
 _workspaces = {}
 
 
@@ -292,8 +299,18 @@ def extract_patches_batch(gray, kpts, count, s_mult, ps=32):
     _need_cuda(gray, "the gray image batch")
     if gray.dtype != torch.uint8:
         raise ValueError("gray images must be uint8 (the /255 is fused into the sampling kernels)")
-    gray, kpts = gray.contiguous(), kpts.contiguous().float()
+    if gray.dim() != 3:
+        raise ValueError("gray images must be [B,H,W], got %s" % (tuple(gray.shape),))
+    _same_device(kpts, gray, "the keypoints")
     B, H, W = gray.shape
+    if kpts.dim() != 3 or kpts.shape[0] != B or kpts.shape[2] != 2:
+        raise ValueError("keypoints must be [B=%d,K,2], got %s" % (B, tuple(kpts.shape)))
+    if count is not None:
+        _same_device(count, gray, "the keypoint counts")
+        if count.shape != (B,) or count.is_floating_point() or count.is_complex():
+            raise ValueError("keypoint counts must be integer [B=%d], got %s %s" % (B, count.dtype, tuple(count.shape)))
+        count = count.contiguous().to(torch.int32)
+    gray, kpts = gray.contiguous(), kpts.contiguous().float()
     K = kpts.shape[1]
     patches = torch.zeros(B, K, ps, ps, dtype=torch.float32, device=gray.device)
     if K == 0:
@@ -332,6 +349,8 @@ def hardnet_forward(patches, packed, precision="tf32"):
         raise ValueError("precision %r is not built (choose from %s)" % (precision, sorted(HARDNET_PRECISIONS)))
     prec = HARDNET_PRECISIONS[precision]
     _need_cuda(patches, "the patches")
+    if patches.dim() != 4 or tuple(patches.shape[1:]) != (1, 32, 32):
+        raise ValueError("patches must be [N,1,32,32], got %s" % (tuple(patches.shape),))
     patches = patches.contiguous().float()
     n = patches.shape[0]
     desc = torch.empty(n, 128, dtype=torch.float32, device=patches.device)
@@ -347,7 +366,13 @@ def hardnet_forward(patches, packed, precision="tf32"):
 def match_smnn(d1, d2, th=0.99, want_dm=False):
     """d1 [n1,128], d2 [n2,128] CUDA -> (dists fp32 [M,1], ids int64 [M,2]) like kornia.feature.match_smnn
     (ids ascending in the first index).  want_dm=True also returns the fp32 distance matrix used."""
-    _need_cuda(d1, "the descriptors")
+    _need_cuda(d1, "the descriptors d1")
+    _same_device(d2, d1, "the descriptors d2")
+    # an empty 1-D array stands for "no descriptors" (demo_match.extract_features returns np.array([]) then)
+    d1, d2 = [d.reshape(0, 128) if d.dim() == 1 and d.numel() == 0 else d for d in (d1, d2)]
+    for name, d in (("d1", d1), ("d2", d2)):
+        if d.dim() != 2 or d.shape[1] != 128 or not d.is_floating_point():
+            raise ValueError("descriptors %s must be floating-point [n,128], got %s %s" % (name, d.dtype, tuple(d.shape)))
     d1, d2 = d1.contiguous().float(), d2.contiguous().float()
     n1, n2 = d1.shape[0], d2.shape[0]
     dev = d1.device
@@ -357,9 +382,8 @@ def match_smnn(d1, d2, th=0.99, want_dm=False):
     dm = torch.empty(n1, n2, dtype=torch.float32, device=dev) if want_dm else None
     nbytes = _match_ws(n1, n2)
     ws = _workspace(dev, nbytes)
-    dim = d1.shape[1] if d1.dim() == 2 and n1 else 128
     with torch.cuda.device(dev):
-        _ok(_match(_ptr(d1), n1, _ptr(d2), n2, int(dim), float(th), _ptr(ids), _ptr(dist), _ptr(cnt), _ptr(dm), _ptr(ws),
+        _ok(_match(_ptr(d1), n1, _ptr(d2), n2, 128, float(th), _ptr(ids), _ptr(dist), _ptr(cnt), _ptr(dm), _ptr(ws),
                    nbytes, _stream(dev)))
     m = int(cnt[0])
     out = (dist[:m].reshape(m, 1), ids[:m].long())

@@ -5,6 +5,7 @@ public demo_match.extract_features / extract_matches chain.
 Floating-point stages carry their tolerance here; match indices are bit-exact given the same
 distance matrix (tie rule: lower index first).  The modules run on CUDA copies of the session fixtures, which stay on
 the CPU for the tests that use them there."""
+import contextlib
 import copy
 
 import numpy as np
@@ -137,6 +138,25 @@ def test_hardnet_rejects_cpu_and_training(hardnet):
 
 
 # ------------------------------------------------------------------------------------------ M1
+MATCH_PATHS = {"tc": 0, "ffma": 1}       # the two distance kernels: 3xTF32 tensor cores, fp32 FFMA (balf_debug_set key 3)
+
+
+@contextlib.contextmanager
+def on_match_path(path):
+    capi().debug_set(3, MATCH_PATHS[path])
+    try:
+        yield path
+    finally:
+        capi().debug_set(3, 0)
+
+
+@pytest.fixture(params=list(MATCH_PATHS))
+def match_path(request):
+    """the M1 tests run on both distance kernels"""
+    with on_match_path(request.param):
+        yield request.param
+
+
 def unit_rows(n, seed, dup_of=None):
     g = torch.Generator().manual_seed(seed)
     d = torch.randn(n, 128, generator=g)
@@ -147,7 +167,7 @@ def unit_rows(n, seed, dup_of=None):
 
 
 @pytest.mark.parametrize("n1,n2", [(2048, 2048), (1000, 777), (65, 300), (2, 2), (2, 9)])
-def test_smnn_bit_exact_on_same_distance_matrix(n1, n2):
+def test_smnn_bit_exact_on_same_distance_matrix(match_path, n1, n2):
     d1 = unit_rows(n1, 1)
     d2 = unit_rows(n2, 2, dup_of=d1)
     dist, ids, dm = capi().match_smnn(d1.to(dev()), d2.to(dev()), 0.99, want_dm=True)
@@ -162,22 +182,27 @@ def test_smnn_bit_exact_on_same_distance_matrix(n1, n2):
 def test_smnn_agreement_with_own_distances():
     d1 = unit_rows(2048, 3)
     d2 = unit_rows(2048, 4, dup_of=d1)
-    _, ids = capi().match_smnn(d1.to(dev()), d2.to(dev()), 0.99)
     _, want = thirdparty.match_smnn(d1, d2, 0.99)
-    a, b = set(map(tuple, ids.cpu().numpy())), set(map(tuple, want.numpy()))
+    b = set(map(tuple, want.numpy()))
     assert len(b) > 500
-    assert len(a & b) / len(b) >= 0.99 and len(a & b) / max(len(a), 1) >= 0.99
+    for path in MATCH_PATHS:
+        with on_match_path(path):
+            _, ids = capi().match_smnn(d1.to(dev()), d2.to(dev()), 0.99)
+        a = set(map(tuple, ids.cpu().numpy()))
+        assert len(a & b) / len(b) >= 0.99 and len(a & b) / max(len(a), 1) >= 0.99, path
 
 
 def test_smnn_ties_and_degenerate():
     d = unit_rows(64, 5)
     d1 = torch.cat([d, d[:8]])                     # duplicated rows -> exactly equal distances
-    dist, ids, dm = capi().match_smnn(d1.to(dev()), d.to(dev()), 0.99, want_dm=True)
-    want_dist, want_ids = thirdparty.match_smnn(d1, d, 0.99, dm=dm.cpu())
-    np.testing.assert_array_equal(ids.cpu().numpy(), want_ids.numpy())
-    for n1, n2 in ((0, 5), (1, 5), (5, 1)):
-        dist, ids = capi().match_smnn(torch.zeros(n1, 128, device=dev()), torch.zeros(n2, 128, device=dev()), 0.99)
-        assert ids.shape == (0, 2) and dist.shape == (0, 1)
+    for path in MATCH_PATHS:
+        with on_match_path(path):
+            dist, ids, dm = capi().match_smnn(d1.to(dev()), d.to(dev()), 0.99, want_dm=True)
+            want_dist, want_ids = thirdparty.match_smnn(d1, d, 0.99, dm=dm.cpu())
+            np.testing.assert_array_equal(ids.cpu().numpy(), want_ids.numpy())
+            for n1, n2 in ((0, 5), (1, 5), (5, 1)):
+                dist, ids = capi().match_smnn(torch.zeros(n1, 128, device=dev()), torch.zeros(n2, 128, device=dev()), 0.99)
+                assert ids.shape == (0, 2) and dist.shape == (0, 1)
 
 
 # ------------------------------------------------------------------------------------------ demo chain
