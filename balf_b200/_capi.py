@@ -543,14 +543,29 @@ _homog_ransac = _sig("balf_find_homography_ransac", c_int, _P, _P, _P, c_int, c_
                      _P, _P, c_size_t, _P)
 
 
-def _ransac(fn_ws, fn, name, p1, p2, count, thr, iters, seed):
+def _pair_inputs(name, p1, p2, count, K):
+    """The shared validation of the RANSAC and pose calls -> (p1, p2 float64 [B,M,2], count int32 [B], K float64 [B,2,9]
+    or None), all contiguous on p1's device.  CPU tensors raise RuntimeError, bad shapes ValueError."""
     _need_cuda(p1, "the matched points")
     _need_cuda(p2, "the matched points")
     _need_cuda(count, "the match counts")
+    if K is not None:
+        _need_cuda(K, "the camera matrices")
     a, b = p1.contiguous().double(), p2.contiguous().double()
     cnt = count.contiguous().to(torch.int32)
     if a.dim() != 3 or a.shape[2] != 2 or b.shape != a.shape or cnt.shape != (a.shape[0],):
         raise ValueError("%s: p1, p2 must be [B,M,2] and count [B]" % name)
+    if K is not None:
+        if K.device != a.device:
+            raise ValueError("%s: K is on %s, expected %s" % (name, K.device, a.device))
+        if not K.is_floating_point() or tuple(K.shape) not in ((a.shape[0], 2, 3, 3), (a.shape[0], 2, 9)):
+            raise ValueError("%s: K must be floating-point [B,2,3,3] or [B,2,9]" % name)
+        K = K.contiguous().double().reshape(a.shape[0], 2, 9)
+    return a, b, cnt, K
+
+
+def _ransac(fn_ws, fn, name, p1, p2, count, thr, iters, seed, K=None):
+    a, b, cnt, k = _pair_inputs(name, p1, p2, count, K)
     B, M, _ = a.shape
     dev = a.device
     out = torch.empty(B, 3, 3, dtype=torch.float64, device=dev)
@@ -558,8 +573,9 @@ def _ransac(fn_ws, fn, name, p1, p2, count, thr, iters, seed):
     n_in = torch.empty(B, dtype=torch.int32, device=dev)
     nbytes = fn_ws(B, M, int(iters))                     # 0 for arguments the call itself rejects
     ws = _workspace(dev, nbytes)
+    kp = () if K is None else (_ptr(k),)
     with torch.cuda.device(dev):
-        _ok(fn(_ptr(a), _ptr(b), _ptr(cnt), B, M, float(thr), int(iters), int(seed) & 0xFFFFFFFFFFFFFFFF, _ptr(out),
+        _ok(fn(_ptr(a), _ptr(b), _ptr(cnt), *kp, B, M, float(thr), int(iters), int(seed) & 0xFFFFFFFFFFFFFFFF, _ptr(out),
                _ptr(mask), _ptr(n_in), _ptr(ws), nbytes, _stream(dev)))
     return out, mask, n_in
 
@@ -580,6 +596,52 @@ def find_fundamental_ransac(p1, p2, count, thr, iters, seed):
     with x2^T F x1 = 0, unit Frobenius norm, inlier mask uint8 [B,M], n_inliers int32 [B]) on the device; RANSAC semantics
     in include/balf_b200.h (balf_find_fundamental_ransac)."""
     return _ransac(_fund_ws, _fund_ransac, "find_fundamental_ransac", p1, p2, count, thr, iters, seed)
+
+
+_ess_ws = _sig("balf_essential_workspace_bytes", c_size_t, c_int, c_int, c_int)
+_ess_ransac = _sig("balf_find_essential_ransac", c_int, _P, _P, _P, _P, c_int, c_int, c_double, c_int, ctypes.c_uint64, _P,
+                   _P, _P, _P, c_size_t, _P)
+_recover_pose = _sig("balf_recover_pose", c_int, _P, _P, _P, _P, _P, _P, c_int, c_int, c_double, _P, _P, _P, _P, _P)
+
+
+def find_essential_ransac(p1, p2, count, K, thr, iters, seed):
+    """p1, p2 float64 [B,M,2] CUDA pixel (x, y) of each pair's matches, count int32 [B] valid rows per pair, K [B,2,3,3]
+    (or [B,2,9]) the camera matrices K1, K2 of each pair on the same device -> (E float64 [B,3,3] with x2'^T E x1' = 0 in
+    calibrated coordinates, unit Frobenius norm, inlier mask uint8 [B,M], n_inliers int32 [B]) on the device; thr in
+    pixels.  RANSAC semantics in include/balf_b200.h (balf_find_essential_ransac)."""
+    return _ransac(_ess_ws, _ess_ransac, "find_essential_ransac", p1, p2, count, thr, iters, seed, K=K)
+
+
+def recover_pose(E, p1, p2, count, K, mask=None, dist_thresh=50.0):
+    """E [B,3,3] (or [B,9]), p1, p2 [B,M,2], count [B] and K [B,2,3,3] (or [B,2,9]) on one CUDA device, mask [B,M] (bool or
+    uint8; None: every valid row) -> (R float64 [B,3,3], t float64 [B,3], pose mask uint8 [B,M], n_good int32 [B]): the
+    pose X2 = R X1 + t of each pair whose candidate puts the most masked matches in front of both cameras
+    (include/balf_b200.h, balf_recover_pose)."""
+    a, b, cnt, k = _pair_inputs("recover_pose", p1, p2, count, K)
+    B, M, _ = a.shape
+    dev = a.device
+    _need_cuda(E, "E")
+    if E.device != dev:
+        raise ValueError("recover_pose: E is on %s, expected %s" % (E.device, dev))
+    if not E.is_floating_point() or tuple(E.shape) not in ((B, 3, 3), (B, 9)):
+        raise ValueError("recover_pose: E must be floating-point [B,3,3] or [B,9]")
+    e = E.contiguous().double()
+    m = None
+    if mask is not None:
+        _need_cuda(mask, "the mask")
+        if mask.device != dev:
+            raise ValueError("recover_pose: mask is on %s, expected %s" % (mask.device, dev))
+        if tuple(mask.shape) != (B, M) or mask.dtype not in (torch.bool, torch.uint8):
+            raise ValueError("recover_pose: mask must be bool or uint8 [B,M]")
+        m = mask.contiguous().to(torch.uint8)
+    R = torch.empty(B, 3, 3, dtype=torch.float64, device=dev)
+    t = torch.empty(B, 3, dtype=torch.float64, device=dev)
+    pmask = torch.empty(B, M, dtype=torch.uint8, device=dev)
+    n_good = torch.empty(B, dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        _ok(_recover_pose(_ptr(e), _ptr(a), _ptr(b), _ptr(cnt), _ptr(k), _ptr(m), B, M, float(dist_thresh), _ptr(R), _ptr(t),
+                          _ptr(pmask), _ptr(n_good), _stream(dev)))
+    return R, t, pmask, n_good
 
 
 _box_nms = _sig("balf_box_nms_map", c_int, _P, c_int, c_int, c_int, c_float, c_float, c_float, c_int, _P, _P, c_size_t, _P)

@@ -31,10 +31,7 @@ constexpr int kModels = 3;               // real roots of the 7-point cubic
 constexpr int kRefitPasses = 8;
 constexpr int kRefitMin = 8;             // the 8-point refit needs 8 inliers
 constexpr int kMaxBisect = 200;
-constexpr int kJacobiSweeps = 32;
-constexpr double kJacobiTol2 = 4.930380657631324e-32;   // 2^-104: off-diagonal sum of squares / diagonal sum of squares
 constexpr int kNormalTerms = 45;         // upper triangle of the 9x9 normal matrix
-constexpr double kInf = __builtin_huge_val();
 
 // F = T2^T Fn T1 with T = [[s, 0, -s cx], [0, s, -s cy], [0, 0, 1]], then unit Frobenius norm with the first
 // largest-magnitude entry positive.  False when the norm is 0 or not finite.
@@ -54,27 +51,14 @@ __device__ __forceinline__ bool denormalise(const double (&Fn)[9], const Norm& n
         F[3 + c] = n.s2 * G[3 + c];
         F[6 + c] = ((ux * G[c]) + (uy * G[3 + c])) + G[6 + c];
     }
-    double s = F[0] * F[0];
-#pragma unroll
-    for (int i = 1; i < 9; ++i) s = s + (F[i] * F[i]);
-    const double nrm = sqrt(s);
-    if (!(nrm > 0.0 && nrm < kInf)) return false;
-#pragma unroll
-    for (int i = 0; i < 9; ++i) F[i] = F[i] / nrm;
-    double big = F[0];
-#pragma unroll
-    for (int i = 1; i < 9; ++i) big = fabs(F[i]) > fabs(big) ? F[i] : big;
-    if (big < 0.0) {
-#pragma unroll
-        for (int i = 0; i < 9; ++i) F[i] = -F[i];
-    }
-    return true;
+    return scale_unit(F);
 }
 
 // Epipolar inlier rule: l2 = F x1 = (a, b, c), s = x2^T l2, l1 = F^T x2 = (a', b', .); both point-to-line distances at
 // most thr, in squared form: s^2 <= thr^2 (a^2 + b^2) and s^2 <= thr^2 (a'^2 + b'^2), each a^2 + b^2 finite and > 0.
 struct Fundamental {
     static constexpr int kMinMatches = kSample;
+    static constexpr bool kPairThr = false;
     static __device__ __forceinline__ bool valid(const double (&F)[9]) {
         bool nz = false;
 #pragma unroll
@@ -93,11 +77,6 @@ struct Fundamental {
         return n2 > 0.0 && n2 < kInf && n1 > 0.0 && n1 < kInf && s2 <= thr2 * n2 && s2 <= thr2 * n1;
     }
 };
-
-__device__ __forceinline__ double det3(const double (&m)[9]) {
-    return ((m[0] * ((m[4] * m[8]) - (m[5] * m[7]))) - (m[1] * ((m[3] * m[8]) - (m[5] * m[6])))) +
-           (m[2] * ((m[3] * m[7]) - (m[4] * m[6])));
-}
 
 __device__ __forceinline__ double poly3(const double (&c)[4], double x) {
     return ((((c[3] * x) + c[2]) * x + c[1]) * x) + c[0];
@@ -255,51 +234,6 @@ __global__ void __launch_bounds__(kHypThreads) fundamental_hyp_kernel(const doub
     for (int m = 0; m < kModels; ++m)
 #pragma unroll
         for (int i = 0; i < 9; ++i) out[9 * m + i] = F[m][i];
-}
-
-// Cyclic Jacobi on the symmetric A (oracle/fundamental.py: jacobi_eigh); V receives the eigenvectors as columns and the
-// return value is the column of the first smallest eigenvalue.
-template <int N>
-__device__ int jacobi_smallest(double (&A)[N][N], double (&V)[N][N]) {
-    for (int i = 0; i < N; ++i)
-        for (int j = 0; j < N; ++j) V[i][j] = i == j ? 1.0 : 0.0;
-    for (int sweep = 0; sweep < kJacobiSweeps; ++sweep) {
-        double off = 0.0, dsq = 0.0;
-        for (int p = 0; p < N; ++p) {
-            dsq = dsq + (A[p][p] * A[p][p]);
-            for (int q = p + 1; q < N; ++q) off = off + (A[p][q] * A[p][q]);
-        }
-        if (!(off > kJacobiTol2 * dsq)) break;
-        for (int p = 0; p < N - 1; ++p)
-            for (int q = p + 1; q < N; ++q) {
-                const double apq = A[p][q];
-                if (apq == 0.0) continue;
-                const double theta = (A[q][q] - A[p][p]) / (2.0 * apq);
-                double t = 1.0 / (fabs(theta) + sqrt((theta * theta) + 1.0));
-                if (theta < 0.0) t = -t;
-                const double c = 1.0 / sqrt((t * t) + 1.0), s = t * c;
-                for (int k = 0; k < N; ++k) {
-                    const double akp = A[k][p], akq = A[k][q];
-                    A[k][p] = (c * akp) - (s * akq);
-                    A[k][q] = (s * akp) + (c * akq);
-                }
-                for (int k = 0; k < N; ++k) {
-                    const double apk = A[p][k], aqk = A[q][k];
-                    A[p][k] = (c * apk) - (s * aqk);
-                    A[q][k] = (s * apk) + (c * aqk);
-                }
-                A[p][q] = 0.0;
-                A[q][p] = 0.0;
-                for (int k = 0; k < N; ++k) {
-                    const double vkp = V[k][p], vkq = V[k][q];
-                    V[k][p] = (c * vkp) - (s * vkq);
-                    V[k][q] = (s * vkp) + (c * vkq);
-                }
-            }
-    }
-    int j = 0;
-    for (int i = 1; i < N; ++i) if (A[i][i] < A[j][j]) j = i;
-    return j;
 }
 
 // The normalised 8-point fit from the 45 normal-matrix sums: the smallest eigenvector f, then F - (F v3) v3^T with v3 the

@@ -67,6 +67,7 @@ __device__ __forceinline__ bool is_inlier(const double (&H)[9], double x1, doubl
 // The model of ransac_score_kernel / mark_inliers (ransac.cuh); H[8] = 0 marks a degenerate hypothesis.
 struct Homography {
     static constexpr int kMinMatches = 4;
+    static constexpr bool kPairThr = false;
     static __device__ __forceinline__ bool valid(const double (&H)[9]) { return H[8] != 0.0; }
     static __device__ __forceinline__ bool inlier(const double (&H)[9], double x1, double y1, double x2, double y2,
                                                   double thr2) {

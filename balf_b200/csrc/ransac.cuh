@@ -1,7 +1,7 @@
-// Pieces shared by the RANSAC estimators (homography.cu, fundamental.cu): the counter-based sampler, the partial-pivot
-// elimination, point normalisation, the chunked scoring kernel with its packed winner key, and the refit kernels'
-// fixed-order block sums.  Both translation units are compiled with -fmad=false, and oracle/homography.py restates every
-// piece (oracle/fundamental.py reuses it).
+// Pieces shared by the RANSAC estimators (homography.cu, fundamental.cu, essential.cu): the counter-based sampler, the
+// partial-pivot elimination, point normalisation, the chunked scoring kernel with its packed winner key, the refit kernels'
+// fixed-order block sums, the unit-norm scaling, det3 and the cyclic Jacobi.  Every translation unit is compiled with
+// -fmad=false, and oracle/homography.py and oracle/fundamental.py restate every piece (oracle/essential.py reuses them).
 #pragma once
 #include "common.cuh"
 
@@ -17,6 +17,9 @@ constexpr int kScoreThreads = 256;
 constexpr int kHypThreads = 128;
 constexpr int kChunk = 1024;             // points per shared-memory chunk of the scoring kernel (32 KB)
 constexpr int kRefitThreads = 256;
+constexpr int kJacobiSweeps = 32;
+constexpr double kJacobiTol2 = 4.930380657631324e-32;   // 2^-104: off-diagonal sum of squares / diagonal sum of squares
+constexpr double kInf = __builtin_huge_val();
 
 __device__ __forceinline__ u64 splitmix64(u64 z) {
     z += 0x9E3779B97F4A7C15ull;
@@ -113,18 +116,21 @@ __device__ __forceinline__ int clamp_count(const int32_t* count, int b, int M) {
 
 // One thread per model slot g (0 <= g < slots) of a pair, 9 doubles each in hyp [B][slots][9]; the pair's points are
 // streamed through shared memory in chunks.  Model supplies kMinMatches (fewer matches: the pair has no model),
-// valid(P) (false for an empty slot) and inlier(P, x1, y1, x2, y2, thr2).
+// kPairThr (true: pair b's squared threshold is thr2_pair[b], not thr2), valid(P) (false for an empty slot) and
+// inlier(P, x1, y1, x2, y2, thr2).
 // key = (inliers + 1) << 32 | (0xFFFFFFFF - g): an empty slot scores -1 (key < 2^32), the maximum key is the highest
 // count, and among equal counts the lowest slot.  Each warp combines its keys and issues one atomicMax into best[b].
 template <class Model>
 __global__ void __launch_bounds__(kScoreThreads) ransac_score_kernel(const double* __restrict__ p1, const double* __restrict__ p2,
                                                                      const int32_t* __restrict__ count, int M, int slots,
                                                                      double thr2, const double* __restrict__ hyp,
-                                                                     u64* __restrict__ best) {
+                                                                     u64* __restrict__ best,
+                                                                     const double* __restrict__ thr2_pair = nullptr) {
     __shared__ double4 pts[kChunk];
     const int g = blockIdx.x * blockDim.x + threadIdx.x, b = blockIdx.y;
     const int n = clamp_count(count, b, M);
     if (n < Model::kMinMatches) return;                              // every slot of the pair is empty
+    if constexpr (Model::kPairThr) thr2 = thr2_pair[b];
     double P[9];
     bool ok = g < slots;
     if (ok) {
@@ -249,6 +255,76 @@ __device__ __forceinline__ int mark_inliers(const double (&G)[9], const double* 
     const int r = *cnt_sh;
     __syncthreads();
     return r;
+}
+
+__device__ __forceinline__ double det3(const double (&m)[9]) {
+    return ((m[0] * ((m[4] * m[8]) - (m[5] * m[7]))) - (m[1] * ((m[3] * m[8]) - (m[5] * m[6])))) +
+           (m[2] * ((m[3] * m[7]) - (m[4] * m[6])));
+}
+
+// F / |F|_F (sum of squares in index order) with its first largest-magnitude entry made positive (oracle/fundamental.py:
+// scale_unit).  False when the norm is 0 or not finite.
+__device__ __forceinline__ bool scale_unit(double (&F)[9]) {
+    double s = F[0] * F[0];
+#pragma unroll
+    for (int i = 1; i < 9; ++i) s = s + (F[i] * F[i]);
+    const double nrm = sqrt(s);
+    if (!(nrm > 0.0 && nrm < kInf)) return false;
+#pragma unroll
+    for (int i = 0; i < 9; ++i) F[i] = F[i] / nrm;
+    double big = F[0];
+#pragma unroll
+    for (int i = 1; i < 9; ++i) big = fabs(F[i]) > fabs(big) ? F[i] : big;
+    if (big < 0.0) {
+#pragma unroll
+        for (int i = 0; i < 9; ++i) F[i] = -F[i];
+    }
+    return true;
+}
+
+// Cyclic Jacobi on the symmetric A (oracle/fundamental.py: jacobi_eigh); V receives the eigenvectors as columns, the
+// diagonal of A the eigenvalues, and the return value is the column of the first smallest eigenvalue.
+template <int N>
+__device__ int jacobi_smallest(double (&A)[N][N], double (&V)[N][N]) {
+    for (int i = 0; i < N; ++i)
+        for (int j = 0; j < N; ++j) V[i][j] = i == j ? 1.0 : 0.0;
+    for (int sweep = 0; sweep < kJacobiSweeps; ++sweep) {
+        double off = 0.0, dsq = 0.0;
+        for (int p = 0; p < N; ++p) {
+            dsq = dsq + (A[p][p] * A[p][p]);
+            for (int q = p + 1; q < N; ++q) off = off + (A[p][q] * A[p][q]);
+        }
+        if (!(off > kJacobiTol2 * dsq)) break;
+        for (int p = 0; p < N - 1; ++p)
+            for (int q = p + 1; q < N; ++q) {
+                const double apq = A[p][q];
+                if (apq == 0.0) continue;
+                const double theta = (A[q][q] - A[p][p]) / (2.0 * apq);
+                double t = 1.0 / (fabs(theta) + sqrt((theta * theta) + 1.0));
+                if (theta < 0.0) t = -t;
+                const double c = 1.0 / sqrt((t * t) + 1.0), s = t * c;
+                for (int k = 0; k < N; ++k) {
+                    const double akp = A[k][p], akq = A[k][q];
+                    A[k][p] = (c * akp) - (s * akq);
+                    A[k][q] = (s * akp) + (c * akq);
+                }
+                for (int k = 0; k < N; ++k) {
+                    const double apk = A[p][k], aqk = A[q][k];
+                    A[p][k] = (c * apk) - (s * aqk);
+                    A[q][k] = (s * apk) + (c * aqk);
+                }
+                A[p][q] = 0.0;
+                A[q][p] = 0.0;
+                for (int k = 0; k < N; ++k) {
+                    const double vkp = V[k][p], vkq = V[k][q];
+                    V[k][p] = (c * vkp) - (s * vkq);
+                    V[k][q] = (s * vkp) + (c * vkq);
+                }
+            }
+    }
+    int j = 0;
+    for (int i = 1; i < N; ++i) if (A[i][i] < A[j][j]) j = i;
+    return j;
 }
 
 inline size_t best_bytes(int B) { return align_up((size_t)B * sizeof(u64), 256); }

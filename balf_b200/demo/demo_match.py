@@ -259,10 +259,33 @@ def extract_matches(args, im_rgb1, im_gray1, im_rgb2, im_gray2, detector, descri
     return kpts1[ids[:, 0], :2], kpts2[ids[:, 1], :2]
 
 
-def _ransac_batch(estimate, name, pairs, ransac_thr, max_iters, seed, device):
-    """The padded batch of ``find_homography_batch`` / ``find_fundamental_batch``: the lists go to the device as one padded
-    float64 buffer, ``estimate`` (a ``_capi`` RANSAC call) runs once, and the 3x3 models and the masks come back in one
-    copy -> [(model [3,3] float64 or None, mask uint8 [M_i,1])]; None where the library returned all zeros (no model)."""
+def _camera_pairs(name, Ks, n):
+    """Ks: n entries, each a 3x3 K (both images) or a pair (K1, K2) -> float64 [n,2,3,3]; ValueError unless every K is
+    3x3 and finite with fx, fy > 0 and last row (0, 0, 1)."""
+    if len(Ks) != n:
+        raise ValueError("%s: %d camera entries for %d pairs" % (name, len(Ks), n))
+    out = np.zeros((n, 2, 3, 3))
+    for i, k in enumerate(Ks):
+        both = isinstance(k, (tuple, list)) and len(k) == 2 and np.ndim(k[0]) == 2
+        a = [np.asarray(x, np.float64) for x in (k if both else (k, k))]
+        if any(x.shape != (3, 3) for x in a):
+            raise ValueError("%s: K of pair %d must be 3x3 or a pair of 3x3" % (name, i))
+        a = np.stack(a)
+        if not (np.isfinite(a).all() and (a[:, 0, 0] > 0).all() and (a[:, 1, 1] > 0).all()
+                and (a[:, 2] == [0.0, 0.0, 1.0]).all()):
+            raise ValueError("%s: K of pair %d must be finite with fx, fy > 0 and last row (0, 0, 1)" % (name, i))
+        out[i] = a
+    return out
+
+
+def _ransac_batch(estimate, name, pairs, ransac_thr, max_iters, seed, device, Ks=None, pose=False):
+    """The padded batch of ``find_homography_batch`` / ``find_fundamental_batch`` / ``find_essential_batch`` /
+    ``relative_pose_batch``: the lists (and the camera matrices Ks, validated first) go to the device as one padded float64
+    buffer, ``estimate`` (a ``_capi`` RANSAC call) runs once, with pose=True ``_capi.recover_pose`` runs on its output on
+    the same stream, and the results come back in one copy -> [(model [3,3] float64 or None, mask uint8 [M_i,1])], with
+    pose=True [(R [3,3] or None, t [3,1] or None, E or None, inlier mask [M_i,1], pose mask [M_i,1])]; None where the
+    library returned all zeros (no model)."""
+    cams = None if Ks is None else _camera_pairs(name, Ks, len(pairs))
     dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
     if not pairs:
         return []
@@ -271,18 +294,40 @@ def _ransac_batch(estimate, name, pairs, ransac_thr, max_iters, seed, device):
         if len(a) != len(b):
             raise ValueError("%s: pts1 and pts2 have %d and %d rows" % (name, len(a), len(b)))
     B, M = len(p), max(max(len(a) for a, _ in p), 1)
-    host = np.zeros(2 * B * M * 2 + B)                    # p1 [B,M,2], p2 [B,M,2], then the counts
+    nk = 0 if cams is None else 18 * B
+    host = np.zeros(2 * B * M * 2 + B + nk)               # p1 [B,M,2], p2 [B,M,2], the counts, then K [B,2,9]
     pts = host[:4 * B * M].reshape(2, B, M, 2)
     for i, (a, b) in enumerate(p):
         pts[0, i, :len(a)], pts[1, i, :len(b)] = a, b
-    host[4 * B * M:] = [len(a) for a, _ in p]
+    host[4 * B * M:4 * B * M + B] = [len(a) for a, _ in p]
+    if cams is not None:
+        host[4 * B * M + B:] = cams.reshape(-1)
     buf = torch.from_numpy(host).to(dev)
     d = buf[:4 * B * M].view(2, B, M, 2)
-    G, mask, _ = estimate(d[0], d[1], buf[4 * B * M:].to(torch.int32), ransac_thr, max_iters, seed)
-    out = torch.cat([G.reshape(-1).view(torch.uint8), mask.reshape(-1)]).cpu().numpy()
+    cnt = buf[4 * B * M:4 * B * M + B].to(torch.int32)
+    kin = () if cams is None else (buf[4 * B * M + B:].view(B, 2, 9),)
+    G, mask, _ = estimate(d[0], d[1], cnt, *kin, ransac_thr, max_iters, seed)
+    parts = [G.reshape(-1).view(torch.uint8), mask.reshape(-1)]
+    if pose:
+        R, t, pmask, _ = _capi.recover_pose(G, d[0], d[1], cnt, kin[0], mask)
+        parts += [R.reshape(-1).view(torch.uint8), t.reshape(-1).view(torch.uint8), pmask.reshape(-1)]
+    out = torch.cat(parts).cpu().numpy()
     Gs = out[:B * 72].view(np.float64).reshape(B, 3, 3)
-    masks = out[B * 72:].reshape(B, M)
-    return [(Gs[i].copy() if Gs[i].any() else None, masks[i, :len(a)].reshape(-1, 1).copy()) for i, (a, _) in enumerate(p)]
+    masks = out[B * 72:B * 72 + B * M].reshape(B, M)
+    if not pose:
+        return [(Gs[i].copy() if Gs[i].any() else None, masks[i, :len(a)].reshape(-1, 1).copy())
+                for i, (a, _) in enumerate(p)]
+    o = B * 72 + B * M
+    Rs = out[o:o + B * 72].view(np.float64).reshape(B, 3, 3)
+    ts = out[o + B * 72:o + B * 96].view(np.float64).reshape(B, 3, 1)
+    pm = out[o + B * 96:].reshape(B, M)
+    res = []
+    for i, (a, _) in enumerate(p):
+        found = Rs[i].any()
+        res.append((Rs[i].copy() if found else None, ts[i].copy() if found else None,
+                    Gs[i].copy() if Gs[i].any() else None, masks[i, :len(a)].reshape(-1, 1).copy(),
+                    pm[i, :len(a)].reshape(-1, 1).copy()))
+    return res
 
 
 def find_homography_batch(pairs, ransac_thr=3.0, max_iters=2000, seed=0, device=None):
@@ -321,3 +366,67 @@ def find_fundamental(pts1, pts2, ransac_thr=3.0, max_iters=1000, seed=0, device=
       returns the best single F.
     Plane degeneracy is not handled: on a planar scene F fits the matches but the epipolar geometry is not determined."""
     return find_fundamental_batch([(pts1, pts2)], ransac_thr, max_iters, seed, device)[0]
+
+
+def find_essential_batch(pairs, Ks, ransac_thr=1.0, max_iters=1000, seed=0, device=None):
+    """RANSAC essential matrices of many calibrated match lists in one library call (semantics: include/balf_b200.h,
+    balf_find_essential_ransac).  pairs = [(pts1 [M_i,2], pts2 [M_i,2])] undistorted pixel coordinates, Ks = one entry per
+    pair, a 3x3 K shared by both images or a pair (K1, K2) -> [(E [3,3] float64 or None, mask uint8 [M_i,1])], each entry
+    in the return layout of ``cv2.findEssentialMat(pts1, pts2, K, cv2.RANSAC, threshold=ransac_thr, maxIters=max_iters)``.
+    E is None when the pair has fewer than 5 matches or no model.  A K that is not 3x3, not finite, has fx or fy <= 0 or a
+    last row other than (0, 0, 1) raises ValueError before anything runs."""
+    return _ransac_batch(_capi.find_essential_ransac, "find_essential", pairs, ransac_thr, max_iters, seed, device, Ks=Ks)
+
+
+def find_essential(pts1, pts2, K1, K2=None, ransac_thr=1.0, max_iters=1000, seed=0, device=None):
+    """GPU counterpart of ``cv2.findEssentialMat(pts1, pts2, K1, cv2.RANSAC, threshold=ransac_thr, maxIters=max_iters)``
+    (and of its two-camera overload when K2 is given) on one match list -> (E [3,3] float64 or None, mask uint8 [M,1]).
+    The differences from cv2:
+    - E is scaled to unit Frobenius norm with its first largest-magnitude entry positive.
+    - The iteration count is fixed (no confidence-driven early exit), so the result is a pure function of (points, K,
+      ransac_thr, max_iters, seed).
+    - With exactly 5 matches cv2 returns every 5-point solution stacked [3k,3]; this returns the best single E."""
+    return find_essential_batch([(pts1, pts2)], [(K1, K1 if K2 is None else K2)], ransac_thr, max_iters, seed, device)[0]
+
+
+def recover_pose(E, pts1, pts2, K1, K2=None, mask=None, dist_thresh=50.0, device=None):
+    """GPU counterpart of ``cv2.recoverPose(E, pts1, pts2, K1, distanceThresh=dist_thresh, mask=mask)`` on one match list
+    -> (n_good, R [3,3], t [3,1], mask uint8 [M,1]), cv2's layout; R, t map camera-1 coordinates to camera 2.  The
+    triangulation is closed-form rather than cv2's SVD (include/balf_b200.h, balf_recover_pose), so a match within rounding
+    of the depth or distance bounds can be counted differently.  An all-zero E gives zeros."""
+    a, b = np.asarray(pts1, np.float64).reshape(-1, 2), np.asarray(pts2, np.float64).reshape(-1, 2)
+    if len(a) != len(b):
+        raise ValueError("recover_pose: pts1 and pts2 have %d and %d rows" % (len(a), len(b)))
+    e = np.asarray(E, np.float64)
+    if e.shape != (3, 3):
+        raise ValueError("recover_pose: E must be 3x3")
+    cams = _camera_pairs("recover_pose", [(K1, K1 if K2 is None else K2)], 1)
+    dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+    n, M = len(a), max(len(a), 1)
+    host = np.zeros(4 * M + 9 + 18)
+    host[:2 * n], host[2 * M:2 * M + 2 * n] = a.reshape(-1), b.reshape(-1)
+    host[4 * M:4 * M + 9], host[4 * M + 9:] = e.reshape(-1), cams.reshape(-1)
+    buf = torch.from_numpy(host).to(dev)
+    m = None
+    if mask is not None:
+        mk = np.asarray(mask).reshape(-1)
+        if len(mk) != n:
+            raise ValueError("recover_pose: mask has %d rows for %d matches" % (len(mk), n))
+        m = torch.zeros(1, M, dtype=torch.uint8)
+        m[0, :n] = torch.from_numpy((mk != 0).astype(np.uint8))
+        m = m.to(dev)
+    cnt = torch.full((1,), n, dtype=torch.int32, device=dev)
+    R, t, pm, ng = _capi.recover_pose(buf[4 * M:4 * M + 9].view(1, 9), buf[:2 * M].view(1, M, 2),
+                                      buf[2 * M:4 * M].view(1, M, 2), cnt, buf[4 * M + 9:].view(1, 2, 9), m, dist_thresh)
+    out = torch.cat([R.reshape(-1).view(torch.uint8), t.reshape(-1).view(torch.uint8), pm.reshape(-1),
+                     ng.view(torch.uint8)]).cpu().numpy()
+    return (int(out[96 + M:].view(np.int32)[0]), out[:72].view(np.float64).reshape(3, 3).copy(),
+            out[72:96].view(np.float64).reshape(3, 1).copy(), out[96:96 + n].reshape(-1, 1).copy())
+
+
+def relative_pose_batch(pairs, Ks, ransac_thr=1.0, max_iters=1000, seed=0, device=None):
+    """Relative poses of many calibrated match lists: ``find_essential_batch`` then ``recover_pose`` on its inliers, both
+    library calls on one stream, with one upload and one download -> [(R [3,3] or None, t [3,1] or None, E [3,3] or None,
+    inlier mask uint8 [M_i,1], pose mask uint8 [M_i,1])]; X2 = R X1 + t with |t| = 1.  None where the pair has no model."""
+    return _ransac_batch(_capi.find_essential_ransac, "relative_pose", pairs, ransac_thr, max_iters, seed, device, Ks=Ks,
+                         pose=True)

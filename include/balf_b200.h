@@ -322,6 +322,68 @@ BALF_API int balf_find_fundamental_ransac(const double* p1, const double* p2, co
                                           int32_t* n_inliers, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Relative pose of calibrated image pairs: RANSAC essential matrix and its decomposition, batched over image pairs.  No
+ * reference counterpart: the semantics are defined here, restated in oracle/essential.py and checked against that
+ * restatement and against cv2.findEssentialMat / cv2.recoverPose.  float64, no fused multiply-add, and only + - * / sqrt
+ * and comparisons, so a result is a pure function of the inputs.
+ * p1, p2 float64 [B,M,2] pixels, count int32 [B] (clamped to [0, M]) as for H and F; K float64 [B,2,9] on the device:
+ * K1 and K2 of each pair, row-major.  Points must already be undistorted.
+ *  - Calibration: y' = (y - cy) / fy, x' = ((x - cx) - s y') / fx with s = K[0,1], each image with its own K.  A pair
+ *    whose K1 or K2 has fx or fy not finite and > 0, or a last row other than (0, 0, 1), gets no model (a per-pair result,
+ *    not an argument error).
+ *  - Threshold: thr in pixels; pair b uses thr_b = thr / f_b, f_b = (((fx1 + fy1) + fx2) + fy2) / 4 (cv2's two-camera
+ *    findEssentialMat divides by the mean focal length in the same way).
+ *  - Sampling: the homography's hash streams unchanged, drawing 5 distinct indices; a hypothesis that has not found them
+ *    after 64 counters has no model.
+ *  - Minimal solver (5-point, Nister / Stewenius): the 4-D null space of the 5x9 system x2'^T E x1' = 0 by one
+ *    partial-pivot elimination of e0..e4 with 4 right-hand sides (e5..e8 free; a pivot that is 0 or not finite: no model),
+ *    orthonormalised by modified Gram-Schmidt in the order W, Z, Y, X (a norm 0 or not finite: no model).  E = xX + yY +
+ *    zZ + W in det E = 0 and E E^T E - (tr(E E^T) / 2) E = 0 gives a 10x20 matrix in the monomials x^3, y^3, x^2y, xy^2,
+ *    x^2z, x^2, y^2z, y^2, xyz, xy, xz^2, xz, x, yz^2, yz, y, z^3, z^2, z, 1 (row 0 the determinant, rows 1 + 3i + j the
+ *    entries (i, j)), reduced by Gauss-Jordan with partial pivoting (first maximum wins; a pivot 0 or not finite: no
+ *    model).  Rows x^2z - z x^2, y^2z - z y^2 and xyz - z xy give B(z) (x, y, 1)^T = 0 with cubic / quartic entries, and
+ *    det B(z) is a degree-10 polynomial.  Its real roots: the degree is the highest one with a finite Cauchy bound R; a
+ *    Sturm sequence (each member divided by its largest-magnitude coefficient) counts the roots in (-R, R], and root i in
+ *    ascending order is bisected on that count (mid = lo / 2 + hi / 2, at most 200 steps; the root is the upper end).
+ *    For root z, (x', y', w') is the cross product of rows 0 and 1 of B(z); w' = 0: no model for that root; x = x' / w',
+ *    y = y' / w'.  Model m (roots ascending) of hypothesis h goes to slot 10 h + m.  No Hartley normalisation (E is not
+ *    invariant to it).
+ *  - Scaling: every E has unit Frobenius norm and its first largest-magnitude entry positive.  A norm of 0 or not finite:
+ *    no model.
+ *  - Inliers (cv2's EMEstimatorCallback error, squared, in calibrated coordinates): with s = x2'^T E x1' and
+ *    d = (E x1')_0^2 + (E x1')_1^2 + (E^T x2')_0^2 + (E^T x2')_1^2, an inlier has d finite and > 0 and s^2 <= thr_b^2 d.
+ *    cv2 rounds s^2 / d to float32; this does not.  The winner is the highest count, the lowest 10 h + m among equal
+ *    counts.  No refit: the output is the winning minimal model and its inliers, as in cv2.findEssentialMat.
+ *  - A pair with fewer than 5 matches, an invalid K or no model: E all zeros, n_inliers = 0, mask all zeros.  With exactly
+ *    5 matches cv2 returns every solution stacked; this returns the best one.
+ * Argument errors (< 0): thr <= 0 (or NaN), iters outside [1, 131072], M outside [0, 16384], B outside [0, 65535], a null
+ * pointer, a workspace smaller than balf_essential_workspace_bytes(B, M, iters).
+ *
+ * balf_recover_pose: E float64 [B,9] (e.g. balf_find_essential_ransac's), p1, p2, count and K as above, mask_in uint8
+ * [B,M] or null (null: every valid row) -> R float64 [B,9] (row-major), t float64 [B,3] (unit), pose_mask uint8 [B,M],
+ * n_good int32 [B].  The pose maps camera-1 coordinates to camera 2: X2 = R X1 + t.
+ *  - Decomposition: V from a 3x3 cyclic Jacobi of E^T E, eigenvalues in descending order (equal ones keep their order);
+ *    u1 = E v1 / |E v1|, u2 = E v2 / |E v2|, u3 = u1 x u2; v3 negated when det V < 0.  R1 = U W V^T, R2 = U W^T V^T with
+ *    W = [[0,-1,0],[1,0,0],[0,0,1]], t = u3.  Candidates in the order (R1, t), (R2, t), (R1, -t), (R2, -t), as
+ *    cv2.recoverPose; which of the two rotations is R1 depends on the signs of the singular vectors, so it can differ
+ *    from cv2.decomposeEssentialMat's R1 (the set is the same).
+ *  - Cheirality: for each masked valid match, (z1, z2) of z2 x2' = z1 R x1' + t by least squares through the 2x2 normal
+ *    equations; with X = z1 x1', the match is good when 0 < z1 < dist_thresh and 0 < (R X + t)_z < dist_thresh.  This is
+ *    cv2's depth and distance test with this closed-form triangulation in place of its SVD-based triangulatePoints, so a
+ *    match within rounding of a bound can be counted differently.
+ *  - Result: the candidate with the most good matches, the first one on ties (cv2's >= chain); pose_mask marks its good
+ *    matches.  An all-zero E, an invalid K or an E whose |E v1| or |E v2| is 0 or not finite: all-zero outputs.
+ * Argument errors (< 0): dist_thresh <= 0 (or NaN), M outside [0, 16384], B outside [0, 65535], a null pointer (mask_in
+ * excepted). */
+BALF_API size_t balf_essential_workspace_bytes(int B, int M, int iters);
+BALF_API int balf_find_essential_ransac(const double* p1, const double* p2, const int32_t* count, const double* K, int B,
+                                        int M, double thr, int iters, uint64_t seed, double* E, uint8_t* inlier_mask,
+                                        int32_t* n_inliers, void* workspace, size_t workspace_bytes, void* stream);
+BALF_API int balf_recover_pose(const double* E, const double* p1, const double* p2, const int32_t* count, const double* K,
+                               const uint8_t* mask_in, int B, int M, double dist_thresh, double* R, double* t,
+                               uint8_t* pose_mask, int32_t* n_good, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * SURVEY.md section 8(e): the one collective of the sharded path.  No reference counterpart (the reference is single-device,
  * demo/demo_match.py:29): image batches are partitioned over the ranks, every rank runs the whole pipeline on its shard, and
  * the fixed-size keypoint records are all-gathered over NCCL (NVLink 5 / NVSwitch).

@@ -1,10 +1,12 @@
-"""RANSAC throughput: balf_find_homography_ransac (--model homography, the default) or balf_find_fundamental_ransac
-(--model fundamental) on the GPU next to cv2.findHomography(RANSAC) / cv2.findFundamentalMat(FM_RANSAC) on the host.
+"""RANSAC throughput: balf_find_homography_ransac (--model homography, the default), balf_find_fundamental_ransac
+(--model fundamental) or balf_find_essential_ransac + balf_recover_pose (--model essential) on the GPU next to
+cv2.findHomography(RANSAC) / cv2.findFundamentalMat(FM_RANSAC) / cv2.findEssentialMat(RANSAC) + cv2.recoverPose on the host.
 
 Workloads: B = 64 synthetic pairs of M = 2048 and M = 8192 matches in a 1200x900 frame with 0.5 px noise, threshold 3 px.
 homography: a seeded homography per pair, inlier ratio 0.3, 2000 hypotheses per pair.  fundamental: a seeded two-view
 scene per pair (3-D points 4 - 10 units in front of camera 1, the second camera rotated by up to 0.1 rad and moved about
-one unit), inlier ratio 0.5, 1000 hypotheses per pair (up to 3 models each).  GPU: warm-up, then CUDA events around enough calls for a window of at least a
+one unit), inlier ratio 0.5, 1000 hypotheses per pair (up to 3 models each).  essential: the same scenes with K given,
+threshold 1 px (cv2's default), 1000 hypotheses per pair (up to 10 models each), then the pose of each pair.  GPU: warm-up, then CUDA events around enough calls for a window of at least a
 second (ms per call, pairs/s), and the library's per-kernel event timing over a second window (kernel time, point
 evaluations B * iters * M per second of kernel time; a fundamental hypothesis counts once although it scores up to 3
 models).  CPU: cv2 over the same pairs, once with its default confidence (0.995 for the homography, 0.99 for the
@@ -12,7 +14,7 @@ fundamental matrix; adaptive iteration count: what a user calls) and once with c
 these inlier ratios: the same work).
 Prints one JSON line per workload with the card name and power limit read in the same run.
 
-    python scripts/homography_bench.py [--model {homography,fundamental}] [--out FILE]
+    python scripts/homography_bench.py [--model {homography,fundamental,essential}] [--out FILE]
 """
 import argparse
 import json
@@ -89,7 +91,7 @@ def time_calls(fn, min_s):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--model", choices=("homography", "fundamental"), default="homography")
+    ap.add_argument("--model", choices=("homography", "fundamental", "essential"), default="homography")
     ap.add_argument("--out", default=None, help="also write the JSON lines to this file")
     ap.add_argument("--min-window", type=float, default=1.0, help="seconds per timed GPU window")
     args = ap.parse_args()
@@ -97,18 +99,28 @@ def main():
     import balf_b200._capi as c
     dev = torch.device("cuda:0")
     name, power = card()
-    fund = args.model == "fundamental"
-    B, thr = 64, 3.0
-    iters, ratio = (1000, 0.5) if fund else (2000, 0.3)
-    synth, estimate, prefix = ((synth_two_view, c.find_fundamental_ransac, "fundamental") if fund else
-                               (synth_pairs, c.find_homography_ransac, "ransac"))
-    conf_default = 0.99 if fund else 0.995
+    fund, ess = args.model == "fundamental", args.model == "essential"
+    B, thr = 64, 1.0 if ess else 3.0
+    iters, ratio = (1000, 0.5) if fund or ess else (2000, 0.3)
+    synth, estimate, prefix = ((synth_two_view, c.find_fundamental_ransac, ("fundamental",)) if fund else
+                               (synth_two_view, None, ("essential", "recover_pose")) if ess else
+                               (synth_pairs, c.find_homography_ransac, ("ransac",)))
+    conf_default = 0.99 if fund else 0.999 if ess else 0.995
+    K = np.array([[800.0, 0, W / 2], [0, 800.0, H / 2], [0, 0, 1]])
     lines = []
     for M in (2048, 8192):
         p1, p2 = synth(M, B, M, ratio)
         d1, d2 = torch.from_numpy(p1).to(dev), torch.from_numpy(p2).to(dev)
         cnt = torch.full((B,), M, dtype=torch.int32, device=dev)
-        call = lambda: estimate(d1, d2, cnt, thr, iters, 0)
+        if ess:
+            Kd = torch.from_numpy(np.tile(K, (B, 2, 1, 1))).to(dev)
+
+            def call():
+                E, mask, n_in = c.find_essential_ransac(d1, d2, cnt, Kd, thr, iters, 0)
+                c.recover_pose(E, d1, d2, cnt, Kd, mask)
+                return E, mask, n_in
+        else:
+            call = lambda: estimate(d1, d2, cnt, thr, iters, 0)
         for _ in range(3):
             call()
         torch.cuda.synchronize()
@@ -123,15 +135,24 @@ def main():
         kernel_ms = sum(kern.values())
         _, _, n_in = call()
         cpu = {}
+        cpu_pairs = 16 if ess else B        # cv2's 5-point RANSAC takes about a second per pair of 8192 matches
         for arm, conf in (("default_confidence", conf_default), ("all_iterations", 1 - 1e-9)):
             t0 = time.perf_counter()
-            if fund:
+            if ess:
+                inl = []
+                for b in range(cpu_pairs):
+                    E, m = cv2.findEssentialMat(p1[b], p2[b], K, cv2.RANSAC, conf, thr, maxIters=iters)
+                    cv2.recoverPose(E[:3], p1[b], p2[b], K, mask=m)
+                    inl.append(int(m.sum()))
+            elif fund:
                 inl = [int(cv2.findFundamentalMat(p1[b], p2[b], cv2.FM_RANSAC, thr, conf, iters)[1].sum()) for b in range(B)]
             else:
                 inl = [int(cv2.findHomography(p1[b], p2[b], cv2.RANSAC, thr, maxIters=iters, confidence=conf)[1].sum())
                        for b in range(B)]
             dt = time.perf_counter() - t0
-            cpu[arm] = {"ms_per_batch": dt * 1e3, "pairs_per_s": B / dt, "mean_inliers": float(np.mean(inl))}
+            cpu[arm] = {"ms_per_batch": dt * 1e3, "pairs_per_s": len(inl) / dt, "mean_inliers": float(np.mean(inl))}
+            if ess:
+                cpu[arm]["pairs"] = len(inl)
         rec = {"model": args.model, "workload": "B=%d M=%d iters=%d ratio=%.1f" % (B, M, iters, ratio), "card": name, "power_limit": power,
                "gpu_ms_per_call": ms, "gpu_calls_timed": n, "gpu_pairs_per_s": B / (ms * 1e-3),
                "kernel_ms": {k: round(v, 4) for k, v in kern.items()}, "kernel_ms_total": kernel_ms,
