@@ -49,6 +49,8 @@ _pad_geometry = _sig("balf_pad_geometry", c_int, c_int, c_int, c_int, *([ctypes.
 _preprocess = _sig("balf_preprocess_u8", c_int, _P, c_int, c_int, c_int, c_int, _P, c_int, c_int, c_int, c_int, _P)
 _det_ws = _sig("balf_detector_workspace_bytes", c_size_t, _arch_p, c_int, c_int, c_int)
 _det_fwd = _sig("balf_detector_forward", c_int, _arch_p, _P, _P, c_int, c_int, c_int, _P, _P, _P, c_size_t, c_int, _P)
+_pad_gray = _sig("balf_pad_gray_u8", c_int, _P, c_int, c_int, c_int, _P, c_int, c_int, c_int, c_int, _P)
+_det_fwd_gray = _sig("balf_detector_forward_gray", c_int, _arch_p, _P, _P, c_int, c_int, c_int, _P, _P, _P, c_size_t, c_int, _P)
 _pixel_shuffle = _sig("balf_pixel_shuffle", c_int, _P, _P, c_int, c_int, c_int, c_int, c_int, _P)
 _nms_ws = _sig("balf_nms_workspace_bytes", c_size_t, c_int, c_int, c_int, c_int)
 _win_nms = _sig("balf_windowed_nms_topk", c_int, _P, *([c_int] * 10), _P, _P, _P, _P, c_size_t, _P)
@@ -177,6 +179,27 @@ def detector_forward(x, packed, arch, precision="fp32", want_logits=True):
     return logits, prob
 
 
+def detector_forward_gray(g, packed, arch, precision="tf32", want_logits=True):
+    """``detector_forward`` for a gray image given as its padded byte plane g [B,Hp,Wp] uint8 (``pad_gray_u8``): bit-identical
+    to ``detector_forward(preprocess_u8(img)[0])``, stage 1 on per-byte tables (balf_detector_forward_gray).  'tf32' only."""
+    _need_cuda(g, "the input")
+    if g.dtype != torch.uint8 or g.dim() != 3:
+        raise ValueError("expected a padded gray byte plane [B, Hp, Wp] uint8, got %s %s" % (g.dtype, tuple(g.shape)))
+    a = arch_struct(arch)
+    g = g.contiguous()
+    B, H, W = g.shape
+    n_logit = arch["cell"] ** 2 + 1
+    logits = torch.empty(B, n_logit, H // arch["cell"], W // arch["cell"], dtype=torch.float32, device=g.device) \
+        if want_logits else None
+    prob = torch.empty(B, H, W, dtype=torch.float32, device=g.device)
+    nbytes = _det_ws(ctypes.byref(a), B, H, W)
+    ws = _workspace(g.device, nbytes)
+    with torch.cuda.device(g.device):
+        _ok(_det_fwd_gray(ctypes.byref(a), _ptr(packed), _ptr(g), B, H, W, _ptr(logits), _ptr(prob), _ptr(ws), nbytes,
+                          PRECISIONS[precision], _stream(g.device)))
+    return logits, prob
+
+
 def pixel_shuffle(t, r):
     _need_cuda(t, "the input")
     t = t.contiguous().float()
@@ -205,6 +228,21 @@ def preprocess_u8(img, factor=64):
     with torch.cuda.device(img.device):
         _ok(_preprocess(_ptr(img), B, H, W, C, _ptr(x), Hp, Wp, top, left, _stream(img.device)))
     return x, (top, left)
+
+
+def pad_gray_u8(img, factor=64):
+    """img [B,H,W,1] uint8 CUDA (gray) -> (g [B,Hp,Wp] uint8, (top, left)): the image bytes in ``preprocess_u8``'s padded
+    geometry, zeros in the padding -- the input of ``detector_forward_gray``."""
+    _need_cuda(img, "the image batch")
+    if img.dtype != torch.uint8 or img.dim() != 4 or img.shape[3] != 1:
+        raise ValueError("expected a gray image batch [B, H, W, 1] uint8, got %s %s" % (img.dtype, tuple(img.shape)))
+    img = img.contiguous()
+    B, H, W, _ = img.shape
+    Hp, Wp, top, left = pad_geometry(H, W, factor)
+    g = torch.empty(B, Hp, Wp, dtype=torch.uint8, device=img.device)
+    with torch.cuda.device(img.device):
+        _ok(_pad_gray(_ptr(img), B, H, W, _ptr(g), Hp, Wp, top, left, _stream(img.device)))
+    return g, (top, left)
 
 
 def _crop_args(score, crop):

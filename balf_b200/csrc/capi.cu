@@ -64,6 +64,25 @@ __global__ void preprocess_u8_kernel(const uint8_t* __restrict__ img, int H, int
         *reinterpret_cast<float4*>(x + (((size_t)b * 3 + c) * Hp + yo) * Wp + xo) = make_float4(v[c][0], v[c][1], v[c][2], v[c][3]);
 }
 
+// the byte-plane form of the same geometry for a gray image: g[b][yo][xo] = the image byte, 0 in the padding.  Sixteen output bytes
+// per thread (Wp is a multiple of 16): one 16-byte store.
+__global__ void pad_gray_u8_kernel(const uint8_t* __restrict__ img, int H, int W, uint8_t* __restrict__ g, int Hp, int Wp, int top,
+                                   int left) {
+    const int xo = 16 * (blockIdx.x * blockDim.x + threadIdx.x), yo = blockIdx.y, b = blockIdx.z;
+    if (xo >= Wp) return;
+    const int yi = yo - top;
+    const bool row_in = yi >= 0 && yi < H;
+    const uint8_t* src = img + ((size_t)b * H + (row_in ? yi : 0)) * W;
+    uint32_t w[4] = {0u, 0u, 0u, 0u};
+#pragma unroll
+    for (int k = 0; k < 16; ++k) {
+        const int xi = xo + k - left;
+        const uint32_t v = row_in && xi >= 0 && xi < W ? src[xi] : 0u;
+        w[k / 4] |= v << (8 * (k % 4));
+    }
+    *reinterpret_cast<uint4*>(g + ((size_t)b * Hp + yo) * Wp + xo) = make_uint4(w[0], w[1], w[2], w[3]);
+}
+
 // tensor_op.py:1-27: out[n, c, r*i+a, r*j+b] = in[n, c*r*r + a*r + b, i, j]
 __global__ void pixel_shuffle_kernel(const float* __restrict__ in, float* __restrict__ out, int C, int H, int W, int r,
                                      size_t total) {
@@ -148,6 +167,21 @@ extern "C" int balf_preprocess_u8(const uint8_t* img, int B, int H, int W, int C
     {
         ProfScope p("preprocess_u8", static_cast<cudaStream_t>(stream));
         preprocess_u8_kernel<<<grid, 128, 0, static_cast<cudaStream_t>(stream)>>>(img, H, W, C, x, Hp, Wp, top, left);
+    }
+    BALF_COUNT_LAUNCH(1);
+    BALF_LAUNCH_OK();
+    return 0;
+}
+
+extern "C" int balf_pad_gray_u8(const uint8_t* img, int B, int H, int W, uint8_t* g, int Hp, int Wp, int top, int left, void* stream) {
+    BALF_REQUIRE(img && g, "null pointer argument");
+    BALF_REQUIRE(B > 0 && H > 0 && W > 0 && top >= 0 && left >= 0 && top + H <= Hp && left + W <= Wp,
+                 "image %dx%d at (%d,%d) does not fit the padded size %dx%d", H, W, top, left, Hp, Wp);
+    BALF_REQUIRE(Hp % 64 == 0 && Wp % 64 == 0, "padded size %dx%d: height and width must be multiples of 64", Hp, Wp);
+    dim3 grid(cdiv(Wp, 16 * 128), Hp, B);
+    {
+        ProfScope p("pad_gray_u8", static_cast<cudaStream_t>(stream));
+        pad_gray_u8_kernel<<<grid, 128, 0, static_cast<cudaStream_t>(stream)>>>(img, H, W, g, Hp, Wp, top, left);
     }
     BALF_COUNT_LAUNCH(1);
     BALF_LAUNCH_OK();

@@ -749,15 +749,18 @@ extern "C" size_t balf_detector_workspace_bytes(const balf_detector_arch* arch, 
     return ws_layout(*arch, chunk_images(*arch, B, Hp, Wp), Hp, Wp, nullptr, nullptr);
 }
 
-extern "C" int balf_detector_forward(const balf_detector_arch* arch, const float* packed, const float* x, int B, int Hp,
-                                     int Wp, float* logits, float* prob, void* workspace, size_t workspace_bytes,
-                                     int precision, void* stream) {
+// the forward of balf_detector_forward (x: fp32 NCHW input) and of balf_detector_forward_gray (g: the padded byte plane of a gray
+// image, stage 1 on the per-byte-table kernels); exactly one of x, g is non-null
+static int detector_forward(const balf_detector_arch* arch, const float* packed, const float* x, const uint8_t* g, int B, int Hp,
+                            int Wp, float* logits, float* prob, void* workspace, size_t workspace_bytes, int precision, void* stream) {
     if (int e = check_arch(arch)) return e;
-    BALF_REQUIRE(packed && x && prob && workspace, "null pointer argument");
+    BALF_REQUIRE(packed && (x || g) && prob && workspace, "null pointer argument");
     BALF_REQUIRE(B > 0 && Hp > 0 && Wp > 0, "B, Hp, Wp must be positive");
     BALF_REQUIRE(Hp % 64 == 0 && Wp % 64 == 0, "input %dx%d: height and width must be multiples of 64 "
                  "(3 max-pools x 8x8 grid/block tokens; pad with mod_padding_symmetric)", Hp, Wp);
     BALF_REQUIRE(precision >= 0 && precision <= 2, "precision %d is not built in this library (0 = fp32, 1 = tf32-class, 2 = f16x3)", precision);
+    BALF_REQUIRE(!g || precision == 1, "gray-input forward: precision %d is not supported (only 1 = tf32-class)", precision);
+    BALF_REQUIRE(!g || (g_tc_mask & 1), "gray-input forward: stage 1 runs on the tensor-core kernels only (debug key 0 bit 0 is clear)");
     const balf_detector_arch& a = *arch;
     const int chunk = chunk_images(a, B, Hp, Wp);
     BALF_REQUIRE(workspace_bytes >= ws_layout(a, chunk, Hp, Wp, nullptr, nullptr), "workspace too small");
@@ -770,14 +773,17 @@ extern "C" int balf_detector_forward(const balf_detector_arch* arch, const float
     if (int e = set_smem(head_kernel<256, 32>, HeadSmem<256, 32>::bytes)) return e;
     for (int b0 = 0; b0 < B; b0 += chunk) {
         const int Bc = B - b0 < chunk ? B - b0 : chunk;
-        const float* xb = x + (size_t)b0 * 3 * Hp * Wp;
+        const float* xb = x ? x + (size_t)b0 * 3 * Hp * Wp : nullptr;
         // precision 1: tensor-core kernels (detector_tc.cu); g_tc_mask (debug hook) can send single
         // stages back to the fp32 kernels -- both paths share the workspace formats.
         const int tcm = precision >= 1 ? g_tc_mask : 0;
         const int px = precision == 2 ? 1 : 0;                 // split precision: fp16 hi + lo operands, three MMAs per product
         const DownW* d = w.down;
         int tiles = 0;
-        if (tcm & 1) {
+        if (g) {
+            if (int e = tc_run_gray_level0(g + (size_t)b0 * Hp * Wp, d[0], a, tc_blob, Bc, Hp, Wp, ws.u, ws.v, ws.r, ws.q, ws.partial, st)) return e;
+            if (int e = run_se<32>(ws, d[0], Bc, Hp * Wp, Hp * Wp / 64, st)) return e;
+        } else if (tcm & 1) {
             if (int e = tc_run_level_dispatch(0, xb, d[0], a, tc_blob, Bc, Hp, Wp, ws.u, ws.v, ws.r, ws.q, ws.partial, st, px, 0)) return e;
             if (int e = run_se<32>(ws, d[0], Bc, Hp * Wp, Hp * Wp / 64, st)) return e;
         } else if (int e = run_level<3, 32, 128, 128>(xb, true, w.down[0], Bc, Hp, Wp, ws, st, &tiles)) return e;
@@ -812,4 +818,18 @@ extern "C" int balf_detector_forward(const balf_detector_arch* arch, const float
         BALF_LAUNCH_OK();
     }
     return 0;
+}
+
+extern "C" int balf_detector_forward(const balf_detector_arch* arch, const float* packed, const float* x, int B, int Hp,
+                                     int Wp, float* logits, float* prob, void* workspace, size_t workspace_bytes,
+                                     int precision, void* stream) {
+    BALF_REQUIRE(x, "null pointer argument");
+    return detector_forward(arch, packed, x, nullptr, B, Hp, Wp, logits, prob, workspace, workspace_bytes, precision, stream);
+}
+
+extern "C" int balf_detector_forward_gray(const balf_detector_arch* arch, const float* packed, const uint8_t* g, int B, int Hp,
+                                          int Wp, float* logits, float* prob, void* workspace, size_t workspace_bytes,
+                                          int precision, void* stream) {
+    BALF_REQUIRE(g, "null pointer argument");
+    return detector_forward(arch, packed, nullptr, g, B, Hp, Wp, logits, prob, workspace, workspace_bytes, precision, stream);
 }

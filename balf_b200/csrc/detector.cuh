@@ -85,5 +85,8 @@ int tc_run_level_dispatch(int level, const float* xin, const DownW& w, const bal
                           int Bc, int h, int wd, float* u, float* v, float* r, float* q, float* partial, cudaStream_t st, int px, int r16);
 int tc_run_head(const float* r, const float* q, const float* scale, const balf_detector_arch& a,
                 const float* blob, int Bc, int hc, int wc, float* logits, float* prob, cudaStream_t st, int px, int r16);
+// stage 1 at precision 1 on g [Bc][h][wd] uint8, the padded byte plane of a gray image (balf_detector_forward_gray)
+int tc_run_gray_level0(const uint8_t* g, const DownW& w, const balf_detector_arch& a, const float* blob, int Bc, int h, int wd,
+                       float* u, float* v, float* r, float* q, float* partial, cudaStream_t st);
 
 }  // namespace balf

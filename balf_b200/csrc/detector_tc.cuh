@@ -942,8 +942,15 @@ __device__ __forceinline__ void conv0_row(const float4 x, const float* vec, int 
 //   C = 64, 128:  two threads per row (two tile groups at C = 64); four threads per row measured no gain
 //   C = 256:      four threads per row: 16 epilogue warps instead of 8 on an SM whose epilogues are latency-bound, -10 %
 // PX = 1: split precision (fp16 hi + lo operands, see BranchG).
-template <int C, int PX> struct BranchCfg {
+// GRAY: the network-input stage on a gray uint8 image (balf_detector_forward_gray).  Every input pixel is one of 256 byte values
+// and everything before the token mixing is a function of the pixel alone, so each CTA tabulates that chain once per byte value
+// (GrayTable) and a tile gathers its rows from the table: only the mixing, gating, dense2 and the residual run per tile.  The
+// mixing accumulator and dense2 share no columns with u / y1 (those come from the table): 2C TMEM columns per group.
+template <int C, int PX, bool GRAY = false> struct BranchCfg {
     static constexpr int TPR = C == 32 ? 1 : C == 256 ? 4 : 2;
+    // GRAY at C = 32 (93 registers, 146 KB of shared memory with the table), ms per step of 64 gray 480x640 images on one B200 at
+    // 1000 W, same-call A/B (scripts/gray_ab.py): 5 groups 11.23, 6 groups (80 registers) 11.22, 7 groups (72 registers, spills)
+    // 11.19 -- inside the noise, so the fp32-input kernel's 5 stays
     static constexpr int groups = C == 32 ? 5 : C == 64 ? 2 : 1;   // tile groups per CTA (shared resident weights)
     static constexpr int NTG = TM * TPR;                           // threads per tile group
     static constexpr int CH = C / TPR;
@@ -954,17 +961,39 @@ template <int C, int PX> struct BranchCfg {
                                                                    // layout of the merge kernel's kind::f16 dense2, half the HBM bytes
     static constexpr int col_u = 0;
     static constexpr int col_y = park_u ? C : 0;
-    static constexpr int ncols = groups * tc_cols(col_y + 2 * C) > 512 ? col_y + 2 * C : tc_cols(col_y + 2 * C);   // TMEM columns per group
+    static constexpr int col_mix = GRAY ? C : col_y + C;           // token-mixing accumulator
+    static constexpr int col_out = GRAY ? 0 : col_y;               // dense2 accumulator
+    static constexpr int ncols = GRAY ? 2 * C : groups * tc_cols(col_y + 2 * C) > 512 ? col_y + 2 * C : tc_cols(col_y + 2 * C);   // TMEM columns per group
     static constexpr uint32_t xch = TPR == 1 ? 0u : 2u * TPR * TM * 8u;   // LayerNorm exchange buffers per group
     static constexpr int SC = TPR == 1 ? 16 : TPR == 4 ? (CH < 32 ? CH : 32) : (CH > 64 ? 64 : CH);   // sub-chunks bound the live registers
 };
+// The per-byte table of the GRAY branch kernels, in shared memory after the carve-up of tc_smem_bytes: [16-byte chunk][256 byte
+// values], chunk-major so that a warp's 16-byte gathers of one chunk stay inside a 4 KB window.  Chunks 0 .. C/4-1: u (fp32, the
+// residual), C/4 .. C/2-1: y1 (fp32, the gating factor), C/2 .. C/2+C/8-1: y2n (the fp16 mixing operand chunks exactly as row_to_a16 wrote them).
+template <int C> struct GrayTable {
+    static constexpr int u0 = 0, y1 = C / 4, y2 = C / 2, chunks = C / 2 + C / 8;
+    static constexpr uint32_t bytes = (uint32_t)chunks * 256u * 16u;
+};
 
-template <int CIN, int C, int BR, int PX>
+// v[0 .. N) = chunks chunk0 .. chunk0 + N / 4 of byte value b of a GrayTable
+template <int N>
+__device__ __forceinline__ void gray_row(const float4* tab, int chunk0, int b, float (&v)[N]) {
+#pragma unroll
+    for (int k = 0; k < N / 4; ++k) {
+        const float4 f = tab[(chunk0 + k) * 256 + b];
+        v[4 * k] = f.x; v[4 * k + 1] = f.y; v[4 * k + 2] = f.z; v[4 * k + 3] = f.w;
+    }
+}
+
+// GRAY: `xin` is the padded byte plane [B][h][w] uint8 (balf_pad_gray_u8) instead of the fp32 NCHW input
+template <int CIN, int C, int BR, int PX, bool GRAY>
 __device__ __forceinline__ void tc_branch_body(const float* __restrict__ xin, const DownW& w, const TcPlan& plan, const UnitGeom& geo,
                                                float* __restrict__ out, float* __restrict__ scratch, unsigned char* smem) {
-    using Cfg = BranchCfg<C, PX>;
+    using Cfg = BranchCfg<C, PX, GRAY>;
     using G = BranchG<CIN, C, PX>;
+    using GT = GrayTable<C>;
     constexpr int CH = Cfg::CH, NG = Cfg::groups, TPR = Cfg::TPR, NTG = Cfg::NTG, SC = Cfg::SC;
+    static_assert(!GRAY || (CIN < 8 && TPR == 1 && PX == 0), "gray mode: network-input stage, one thread per row, single-rounded operands");
     constexpr bool X3 = PX != 0;
     constexpr int LOC = X3 ? C / 8 : 0;                                   // lo chunks of an A operand follow its C / 8 hi chunks
     constexpr bool XH = !X3 && CIN >= 8;                                  // the level input arrives as fp16 (pool_kernel, single-rounded path)
@@ -1030,47 +1059,14 @@ __device__ __forceinline__ void tc_branch_body(const float* __restrict__ xin, co
         upk2(s2, a, b); sum = a + b;
         upk2(q2, a, b); sq = a + b;
     };
-    // (the coordinates of the prefetched tile are carried into its iteration: the unit -> pixel arithmetic ran twice per tile)
-    bool nvld = false; int nim = 0, npx = 0;
-    if (InputPf<CIN, TPR>::enabled && vblock < ntiles) {
-        coords(vblock, nvld, nim, npx);
-        fetch_input_row<CIN, true, TPR, XH>(xin, npix, (size_t)nim, npx, nvld, half, pf);
-    }
-    for (int t = vblock; t < ntiles; t += vgrid, ++it) {
-        TC_TRACE(plan, it, 0);
-        bool valid; int img, pix;
-        if (InputPf<CIN, TPR>::enabled && (TPR > 1 || !X3)) { valid = nvld; img = nim; pix = npx; }   // (split precision at one thread per row: no registers to spare)
-        else coords(t, valid, img, pix);
-        float* orow = rt + ((size_t)img * npix + pix) * C + col0;
-        float v[CH], rstd, shift;
-        // ---- x -> conv.0 -> ReLU -> LayerNorm (affine folded into dense1)
-        if constexpr (CIN < 8) {
-            const float4 xv = pf.v[0];
-            if (t + vgrid < ntiles) {
-                coords(t + vgrid, nvld, nim, npx);
-                fetch_input_row<CIN, true, TPR, XH>(xin, npix, (size_t)nim, npx, nvld, half, pf);
-            }
-            conv0_row<CIN, C, CH>(xv, s.vec, col0, v);
-        } else {
-            if (InputPf<CIN, TPR>::enabled) {
-                store_input_row<CIN, true, TPR, XM>(pf, s.region, row, half);
-                if (t + vgrid < ntiles) {
-                    coords(t + vgrid, nvld, nim, npx);
-                    fetch_input_row<CIN, true, TPR, XH>(xin, npix, (size_t)nim, npx, nvld, half, pf);
-                }
-            } else {
-                load_input_row<CIN, TPR, XM>(xin, npix, (size_t)img, pix, valid, s.region, row, half);
-            }
-            TC_TRACE(plan, it, 1);
-            sync_for_mma<NG, NTG>(grp);
-            if (w0 && elect_one()) { issue_linear_t<G, BG_CONV0>(ring, plan, region_addr, ones_addr, tm + Cfg::col_y, true); commit(s.done); }
-            TC_TRACE(plan, it, 2);
-            wait_done_ring<G, NG, NTG>(s.done, phase, ring, plan, w0, grp);
-            TC_TRACE(plan, it, 3);
-            ld_row<CH>(lane_base + Cfg::col_y + col0, v);
-#pragma unroll
-            for (int i = 0; i < CH; ++i) v[i] = fmaxf(v[i], 0.f);
-        }
+    // ---- the pixel-local chain before the token mixing: v = x0 = ReLU(conv.0(x)) of this thread's part of the row -> LayerNorm
+    // (affine folded into dense1) -> this branch's half of dense1 -> GELU = u (the residual: parked at col_u, or stored to `rt`)
+    // -> LayerNorm (affine folded into gMLP dense1) -> gMLP dense1 (two halves) -> GELU: y1 parked at col_y, y2 -> LayerNorm ->
+    // affine -> the fp16 mixing operand in the region.  `tmb`: TMEM base of the accumulators.  Every step is row-local, so the
+    // GRAY table build below runs this same code on rows whose inputs are the 256 byte values.
+    auto pre_mix = [&](float (&v)[CH], uint32_t tmb, bool valid, int img, int pix) {
+        const uint32_t lb = tmb + ((uint32_t)(row & ~31) << 16);
+        float rstd, shift;
         {
             float sum, sq;
             stats_of(v, sum, sq);
@@ -1081,15 +1077,15 @@ __device__ __forceinline__ void tc_branch_body(const float* __restrict__ xin, co
         TC_TRACE(plan, it, 4);
         sync_for_mma<NG, NTG>(grp);
         // ---- this branch's half of dense1 -> GELU = u (residual, parked) -> LayerNorm (affine folded into gMLP dense1)
-        if (w0 && elect_one()) { issue_linear_t<G, BG_PD1>(ring, plan, region_addr, ones_addr, tm + Cfg::col_u, true); commit(s.done); }
+        if (w0 && elect_one()) { issue_linear_t<G, BG_PD1>(ring, plan, region_addr, ones_addr, tmb + Cfg::col_u, true); commit(s.done); }
         TC_TRACE(plan, it, 5);
         wait_done_ring<G, NG, NTG>(s.done, phase, ring, plan, w0, grp);
         TC_TRACE(plan, it, 6);
         {
-            ld_row<CH>(lane_base + Cfg::col_u + col0, v);
+            ld_row<CH>(lb + Cfg::col_u + col0, v);
             float sum = 0.f, sq = 0.f;
             gelu_row<CH, true>(v, sum, sq);
-            if (Cfg::park_u) st_row<CH>(lane_base + Cfg::col_u + col0, v);
+            if (Cfg::park_u) st_row<CH>(lb + Cfg::col_u + col0, v);
             else if constexpr (CH % 32 == 0 && !X3) oct_store<CH / 4>(rt, ((size_t)img * npix + pix) * C + col0, ostride, v, valid);
             else pair_store<CH / 4>(rt, ((size_t)img * npix + pix) * C + col0, v, valid);
             row_stats<NG, TPR>(sum, sq, s.xch + (xb++ & 1) * TPR * TM, row, half, C, rstd, shift, grp);
@@ -1100,18 +1096,18 @@ __device__ __forceinline__ void tc_branch_body(const float* __restrict__ xin, co
         sync_for_mma<NG, NTG>(grp);
         // ---- gMLP dense1 (two halves) -> GELU; y1 parked, y2 -> LayerNorm -> [channel][token] operand
         if (w0 && elect_one()) {
-            issue_linear_t<G, BG_D1A>(ring, plan, region_addr, ones_addr, tm + Cfg::col_y, true);
-            issue_linear_t<G, BG_D1B>(ring, plan, region_addr, ones_addr, tm + Cfg::col_y + C, true);
+            issue_linear_t<G, BG_D1A>(ring, plan, region_addr, ones_addr, tmb + Cfg::col_y, true);
+            issue_linear_t<G, BG_D1B>(ring, plan, region_addr, ones_addr, tmb + Cfg::col_y + C, true);
             commit(s.done);
         }
         TC_TRACE(plan, it, 8);
         wait_done_ring<G, NG, NTG>(s.done, phase, ring, plan, w0, grp);
         TC_TRACE(plan, it, 9);
         {
-            ld_row<CH>(lane_base + Cfg::col_y + col0, v);
+            ld_row<CH>(lb + Cfg::col_y + col0, v);
             { float d0, d1; gelu_row<CH, false>(v, d0, d1); }
-            st_row<CH>(lane_base + Cfg::col_y + col0, v);
-            ld_row<CH>(lane_base + Cfg::col_y + C + col0, v);
+            st_row<CH>(lb + Cfg::col_y + col0, v);
+            ld_row<CH>(lb + Cfg::col_y + C + col0, v);
             float sum = 0.f, sq = 0.f;
             gelu_row<CH, true>(v, sum, sq);
             row_stats<NG, TPR>(sum, sq, s.xch + (xb++ & 1) * TPR * TM, row, half, C, rstd, shift, grp);
@@ -1124,10 +1120,97 @@ __device__ __forceinline__ void tc_branch_body(const float* __restrict__ xin, co
             }
             row_to_a16<CH, LOC>(v, s.region, row, col0);          // the mixing MMA reads it as an MN-major B operand (issue_mix_t)
         }
+    };
+    // GRAY: byte value g of the input plane (padding and units past the end read as 0, like the zeros of the fp32 input)
+    const uint8_t* const gin = reinterpret_cast<const uint8_t*>(xin);
+    const float4* const gtab = reinterpret_cast<const float4*>(smem + tc_smem_bytes(Cfg::region, plan, NG, Cfg::xch));
+    int nbyte = 0;
+    if constexpr (GRAY) {
+        // Table build: groups 0 and 1 each run one tile whose rows are the byte values g = 128 grp + row, from balf_preprocess_u8's
+        // input value float(g) / 255 in all three planes, through conv.0 and pre_mix -- the same code the fp32-input kernel runs per
+        // pixel, so every entry is bit-identical to what that kernel computes for a pixel of value g.  Each group builds in TMEM
+        // columns 3C apart (the main loop's 2C-column layout is not in use yet).
+        static_assert(NG >= 2 && 2 * 3 * C <= tc_cols(Cfg::ncols * NG), "gray table build: two groups, 3C TMEM columns each");
+        if (grp < 2) {
+            const int g = grp * TM + row;
+            const float x = (float)g / 255.0f;
+            float v[CH];
+            conv0_row<CIN, C, CH>(make_float4(x, x, x, 0.f), s.vec, col0, v);
+            const uint32_t tmb = *s.tmem_slot + (uint32_t)(grp * 3 * C);
+            pre_mix(v, tmb, false, 0, 0);
+            float4* const tab = const_cast<float4*>(gtab);
+            const uint32_t lb = tmb + ((uint32_t)(row & ~31) << 16);
+            ld_row<CH>(lb + Cfg::col_u, v);
+#pragma unroll
+            for (int k = 0; k < C / 4; ++k) tab[(GT::u0 + k) * 256 + g] = make_float4(v[4 * k], v[4 * k + 1], v[4 * k + 2], v[4 * k + 3]);
+            ld_row<CH>(lb + Cfg::col_y, v);
+#pragma unroll
+            for (int k = 0; k < C / 4; ++k) tab[(GT::y1 + k) * 256 + g] = make_float4(v[4 * k], v[4 * k + 1], v[4 * k + 2], v[4 * k + 3]);
+#pragma unroll
+            for (int j = 0; j < C / 8; ++j) tab[(GT::y2 + j) * 256 + g] = *reinterpret_cast<const float4*>(s.region + ((size_t)j * TM + row) * 4);
+        }
+        fence_before_sync();
+        __syncthreads();
+        fence_after_sync();
+    }
+    // (the coordinates of the prefetched tile are carried into its iteration: the unit -> pixel arithmetic ran twice per tile)
+    bool nvld = false; int nim = 0, npx = 0;
+    if (InputPf<CIN, TPR>::enabled && vblock < ntiles) {
+        coords(vblock, nvld, nim, npx);
+        if constexpr (GRAY) nbyte = nvld ? __ldg(gin + (size_t)nim * npix + npx) : 0;
+        else fetch_input_row<CIN, true, TPR, XH>(xin, npix, (size_t)nim, npx, nvld, half, pf);
+    }
+    for (int t = vblock; t < ntiles; t += vgrid, ++it) {
+        TC_TRACE(plan, it, 0);
+        bool valid; int img, pix;
+        if (InputPf<CIN, TPR>::enabled && (TPR > 1 || !X3)) { valid = nvld; img = nim; pix = npx; }   // (split precision at one thread per row: no registers to spare)
+        else coords(t, valid, img, pix);
+        float* orow = rt + ((size_t)img * npix + pix) * C + col0;
+        const int gv = nbyte;                                  // GRAY: this row's byte value
+        if constexpr (GRAY) {
+            if (t + vgrid < ntiles) {
+                coords(t + vgrid, nvld, nim, npx);
+                nbyte = nvld ? __ldg(gin + (size_t)nim * npix + npx) : 0;
+            }
+            // y2n of the byte -> the mixing operand
+#pragma unroll
+            for (int j = 0; j < C / 8; ++j) *reinterpret_cast<float4*>(s.region + ((size_t)j * TM + row) * 4) = gtab[(GT::y2 + j) * 256 + gv];
+        } else {
+            float v[CH];
+            // ---- x -> conv.0 -> ReLU
+            if constexpr (CIN < 8) {
+                const float4 xv = pf.v[0];
+                if (t + vgrid < ntiles) {
+                    coords(t + vgrid, nvld, nim, npx);
+                    fetch_input_row<CIN, true, TPR, XH>(xin, npix, (size_t)nim, npx, nvld, half, pf);
+                }
+                conv0_row<CIN, C, CH>(xv, s.vec, col0, v);
+            } else {
+                if (InputPf<CIN, TPR>::enabled) {
+                    store_input_row<CIN, true, TPR, XM>(pf, s.region, row, half);
+                    if (t + vgrid < ntiles) {
+                        coords(t + vgrid, nvld, nim, npx);
+                        fetch_input_row<CIN, true, TPR, XH>(xin, npix, (size_t)nim, npx, nvld, half, pf);
+                    }
+                } else {
+                    load_input_row<CIN, TPR, XM>(xin, npix, (size_t)img, pix, valid, s.region, row, half);
+                }
+                TC_TRACE(plan, it, 1);
+                sync_for_mma<NG, NTG>(grp);
+                if (w0 && elect_one()) { issue_linear_t<G, BG_CONV0>(ring, plan, region_addr, ones_addr, tm + Cfg::col_y, true); commit(s.done); }
+                TC_TRACE(plan, it, 2);
+                wait_done_ring<G, NG, NTG>(s.done, phase, ring, plan, w0, grp);
+                TC_TRACE(plan, it, 3);
+                ld_row<CH>(lane_base + Cfg::col_y + col0, v);
+#pragma unroll
+                for (int i = 0; i < CH; ++i) v[i] = fmaxf(v[i], 0.f);
+            }
+            pre_mix(v, tm, valid, img, pix);
+        }
         TC_TRACE(plan, it, 10);
         sync_for_mma<NG, NTG>(grp);
         // ---- token mixing, gating y1 * (y2' + 1)
-        if (w0 && elect_one()) { issue_mix_t<G, BG_WM, C>(ring, plan, region_addr, tm + Cfg::col_y + C); commit(s.done); }
+        if (w0 && elect_one()) { issue_mix_t<G, BG_WM, C>(ring, plan, region_addr, tm + Cfg::col_mix); commit(s.done); }
         TC_TRACE(plan, it, 11);
         wait_done_ring<G, NG, NTG>(s.done, phase, ring, plan, w0, grp);
         TC_TRACE(plan, it, 12);
@@ -1135,8 +1218,9 @@ __device__ __forceinline__ void tc_branch_body(const float* __restrict__ xin, co
 #pragma unroll 1
             for (int c = 0; c < CH; c += SC) {
                 float y1[SC], y2[SC];
-                ld_row<SC>(lane_base + Cfg::col_y + col0 + c, y1);
-                ld_row<SC>(lane_base + Cfg::col_y + C + col0 + c, y2);
+                if constexpr (GRAY) gray_row<SC>(gtab, GT::y1 + (col0 + c) / 4, gv, y1);
+                else ld_row<SC>(lane_base + Cfg::col_y + col0 + c, y1);
+                ld_row<SC>(lane_base + Cfg::col_mix + col0 + c, y2);
                 const float mix_b1 = *mix_b1p;
                 const unsigned long long b2 = pk2(mix_b1, mix_b1);
 #pragma unroll
@@ -1147,7 +1231,7 @@ __device__ __forceinline__ void tc_branch_body(const float* __restrict__ xin, co
         TC_TRACE(plan, it, 13);
         sync_for_mma<NG, NTG>(grp);
         // ---- dense2 + residual u -> out
-        if (w0 && elect_one()) { issue_linear_t<G, BG_D2>(ring, plan, region_addr, ones_addr, tm + Cfg::col_y, true); commit(s.done); }
+        if (w0 && elect_one()) { issue_linear_t<G, BG_D2>(ring, plan, region_addr, ones_addr, tm + Cfg::col_out, true); commit(s.done); }
         TC_TRACE(plan, it, 14);
         wait_done_ring<G, NG, NTG>(s.done, phase, ring, plan, w0, grp);
         TC_TRACE(plan, it, 15);
@@ -1167,7 +1251,7 @@ __device__ __forceinline__ void tc_branch_body(const float* __restrict__ xin, co
 #pragma unroll
                 for (int c = 0; c < CH; c += SC) {
                     float a[SC];
-                    ld_row<SC>(lane_base + Cfg::col_y + col0 + c, a);
+                    ld_row<SC>(lane_base + Cfg::col_out + col0 + c, a);
 #pragma unroll
                     for (int j0 = 0; j0 < SC / 4; j0 += 8) {
                         float4 t8[8];
@@ -1193,8 +1277,9 @@ __device__ __forceinline__ void tc_branch_body(const float* __restrict__ xin, co
 #pragma unroll 1
             for (int c = 0; c < CH; c += SC) {
                 float a[SC], r[SC];
-                ld_row<SC>(lane_base + Cfg::col_y + col0 + c, a);
-                if (Cfg::park_u) ld_row<SC>(lane_base + Cfg::col_u + col0 + c, r);
+                ld_row<SC>(lane_base + Cfg::col_out + col0 + c, a);
+                if constexpr (GRAY) gray_row<SC>(gtab, GT::u0 + (col0 + c) / 4, gv, r);
+                else if (Cfg::park_u) ld_row<SC>(lane_base + Cfg::col_u + col0 + c, r);
                 if constexpr (Cfg::h16_out) {
                     // fp16 tile of the merge kernel: chunk j (8 channels) of pixel row p sits at halves j * 1024 + p * 8 of the
                     // tile; a lane stores 16 bytes per chunk -- neighbouring pixels (the other unit of the tile in the grid
@@ -1264,11 +1349,11 @@ __device__ __forceinline__ void tc_branch_body(const float* __restrict__ xin, co
     tc_finish(*s.tmem_slot, tc_cols(Cfg::ncols * NG));
 }
 
-template <int CIN, int C, int BR, int PX>
-__global__ void __launch_bounds__(BranchCfg<C, PX>::NTG * BranchCfg<C, PX>::groups, 1)
+template <int CIN, int C, int BR, int PX, bool GRAY>
+__global__ void __launch_bounds__(BranchCfg<C, PX, GRAY>::NTG * BranchCfg<C, PX, GRAY>::groups, 1)
 tc_branch_kernel(const float* __restrict__ xin, DownW w, TcPlan plan, UnitGeom geo, float* __restrict__ out, float* __restrict__ scratch) {
     extern __shared__ __align__(1024) unsigned char smem[];
-    tc_branch_body<CIN, C, BR, PX>(xin, w, plan, geo, out, scratch, smem);
+    tc_branch_body<CIN, C, BR, PX, GRAY>(xin, w, plan, geo, out, scratch, smem);
 }
 
 
@@ -1586,7 +1671,9 @@ template <int CIN, int C, int PX = 0> struct MergeBulkCfg {
     static constexpr int min_ctas = C <= 32 ? (PX ? 2 : kMerge32Ctas) : 1;
 };
 
-template <int CIN, int C, int PX = 0>
+// GRAY (stage 1 on a gray uint8 image): `xin` is the padded byte plane [B][h][w] (balf_pad_gray_u8); x = float(g) / 255 in all
+// three planes, as balf_preprocess_u8 computes it, so conv.0 sees the values of the fp32-input kernel bit for bit
+template <int CIN, int C, int PX = 0, bool GRAY = false>
 __global__ void __launch_bounds__(NT2, MergeBulkCfg<CIN, C, PX>::min_ctas)
 tc_merge_bulk_kernel(const float* __restrict__ xin, DownW w, TcPlan plan, UnitGeom geo, const float* __restrict__ uin,
                      const float* __restrict__ vin, float* __restrict__ rout, float* __restrict__ qout, float* __restrict__ partial) {
@@ -1631,10 +1718,19 @@ tc_merge_bulk_kernel(const float* __restrict__ xin, DownW w, TcPlan plan, UnitGe
         bulk_load(v_addr, vin + (size_t)tt * (Cfg::uv_bytes / 4), Cfg::uv_bytes, ld_bar);
     };
     InputPf<CIN> pfx;
+    int pbyte = 0;                                          // GRAY: the prefetched byte (converted where it is used, not where it lands)
+    auto fetch_x = [&](int im, int px) {
+        if constexpr (GRAY) {
+            static_assert(Cfg::cc0 && PX == 0, "gray mode: network-input stage, single-rounded operands");
+            pbyte = __ldg(reinterpret_cast<const uint8_t*>(xin) + (size_t)im * npix + px);
+        } else {
+            fetch_input_row<CIN, false, 2, XH>(xin, npix, (size_t)im, px, true, half, pfx);
+        }
+    };
     if ((int)blockIdx.x < ntiles) {
         int im, px;
         coords(blockIdx.x, im, px);
-        fetch_input_row<CIN, false, 2, XH>(xin, npix, (size_t)im, px, true, half, pfx);
+        fetch_x(im, px);
         if (w0 && elect_one()) load_tile(blockIdx.x);
     }
     for (int t = blockIdx.x; t < ntiles; t += gridDim.x) {
@@ -1655,11 +1751,16 @@ tc_merge_bulk_kernel(const float* __restrict__ xin, DownW w, TcPlan plan, UnitGe
             bulk_wait_read();                               // the previous tile's q / r stores have left W and Q
         }
         ++ld_phase;
-        if constexpr (Cfg::cc0) conv0_row<CIN, C, CH>(pfx.v[0], s.vec, col0, x0);
+        if constexpr (GRAY) {
+            const float x = (float)pbyte / 255.0f;
+            conv0_row<CIN, C, CH>(make_float4(x, x, x, 0.f), s.vec, col0, x0);
+        } else if constexpr (Cfg::cc0) {
+            conv0_row<CIN, C, CH>(pfx.v[0], s.vec, col0, x0);
+        }
         if (nt < ntiles) {
             int im, px;
             coords(nt, im, px);
-            fetch_input_row<CIN, false, 2, XH>(xin, npix, (size_t)im, px, true, half, pfx);
+            fetch_x(im, px);
         }
         wait_done_ring<G>(s.done, phase, ring, plan, w0);
         // x1 = acc + x0; q = x1 + x0 -> Q (staging); LayerNorm(x1) (affine folded into conv1) -> W
@@ -2190,29 +2291,30 @@ static int tc_launch_cfg(K kernel, size_t smem, int tmem_cols, int ntiles, int* 
 }
 
 
-template <int CIN, int C, int PX>
+template <int CIN, int C, int PX, bool GRAY>
 static int tc_launch_branches(const float* xin, const DownW& w, const TcPlans& P, int level, const UnitGeom& g, int ntiles,
                               float* u, float* v, float* su, float* sv, cudaStream_t st) {
-    using Cfg = BranchCfg<C, PX>;
+    using Cfg = BranchCfg<C, PX, GRAY>;
     constexpr int NG = Cfg::groups;
     int grid = 0;
     for (int b = 0; b < 2; ++b) {
         const TcPlan& p = P.branch[level][b];
-        const size_t smem = tc_smem_bytes(Cfg::region, p, NG, Cfg::xch);
+        const size_t smem = tc_smem_bytes(Cfg::region, p, NG, Cfg::xch) + (GRAY ? GrayTable<C>::bytes : 0u);   // + the table (GRAY)
         if (b == 0) {
-            if (int e = tc_launch_cfg(tc_branch_kernel<CIN, C, 0, PX>, smem, tc_cols(Cfg::ncols * NG), ntiles, &grid, NG, Cfg::NTG)) return e;
+            if (int e = tc_launch_cfg(tc_branch_kernel<CIN, C, 0, PX, GRAY>, smem, tc_cols(Cfg::ncols * NG), ntiles, &grid, NG, Cfg::NTG)) return e;
             ProfScope ps(C == 32 ? "det_branch_grid_c32" : C == 64 ? "det_branch_grid_c64" : C == 128 ? "det_branch_grid_c128" : "det_branch_grid_c256", st);
-            tc_branch_kernel<CIN, C, 0, PX><<<grid, Cfg::NTG * NG, smem, st>>>(xin, w, p, g, u, su);
+            tc_branch_kernel<CIN, C, 0, PX, GRAY><<<grid, Cfg::NTG * NG, smem, st>>>(xin, w, p, g, u, su);
         } else {
-            if (int e = tc_launch_cfg(tc_branch_kernel<CIN, C, 1, PX>, smem, tc_cols(Cfg::ncols * NG), ntiles, &grid, NG, Cfg::NTG)) return e;
+            if (int e = tc_launch_cfg(tc_branch_kernel<CIN, C, 1, PX, GRAY>, smem, tc_cols(Cfg::ncols * NG), ntiles, &grid, NG, Cfg::NTG)) return e;
             ProfScope ps(C == 32 ? "det_branch_block_c32" : C == 64 ? "det_branch_block_c64" : C == 128 ? "det_branch_block_c128" : "det_branch_block_c256", st);
-            tc_branch_kernel<CIN, C, 1, PX><<<grid, Cfg::NTG * NG, smem, st>>>(xin, w, p, g, v, sv);
+            tc_branch_kernel<CIN, C, 1, PX, GRAY><<<grid, Cfg::NTG * NG, smem, st>>>(xin, w, p, g, v, sv);
         }
     }
     return 0;
 }
 
-template <int CIN, int C, int PX>
+// GRAY: stage 1 on the padded byte plane of a gray image (`xin` points at uint8 data, see tc_run_gray_level0)
+template <int CIN, int C, int PX, bool GRAY = false>
 static int tc_run_level(const float* xin, const DownW& w, const TcPlans& P, int level, int Bc, int h, int wd,
                         float* u, float* v, float* r, float* q, float* partial, cudaStream_t st, int r16) {
     UnitGeom g{h, wd, h / 8, wd / 8, h * wd / 64, Bc * (h * wd / 64), 1.0f / (float)(h * wd / 64), 1.0f / (float)(wd / 8), 1.0f / (float)(wd / 8)};
@@ -2222,14 +2324,14 @@ static int tc_run_level(const float* xin, const DownW& w, const TcPlans& P, int 
     BALF_REQUIRE((plan_matches<BranchG<CIN, C, PX>>(P.branch[level][0]) && plan_matches<BranchG<CIN, C, PX>>(P.branch[level][1]) &&
                   plan_matches<MergeG<CIN, C, PX>>(P.merge[level])), "internal: compile-time and packed GEMM plans differ (level %d)", level);
     // (r and q are free until the merge kernel writes them: scratch of the stage-4 branch kernels' residual round trip)
-    if (int e = tc_launch_branches<CIN, C, PX>(xin, w, P, level, g, ntiles, u, v, r, q, st)) return e;
+    if (int e = tc_launch_branches<CIN, C, PX, GRAY>(xin, w, P, level, g, ntiles, u, v, r, q, st)) return e;
     if constexpr (C <= 64) {
         const TcPlan& p = P.merge[level];
         BALF_REQUIRE(g.total_units % 2 == 0, "internal: odd unit count at stage %d", level);
         const size_t smem = tc_smem_bytes(MergeBulkCfg<CIN, C, PX>::region, p, 1, MergeBulkCfg<CIN, C, PX>::xch);
-        if (int e = tc_launch_cfg(tc_merge_bulk_kernel<CIN, C, PX>, smem, MergeBulkCfg<CIN, C, PX>::ncols, ntiles, &grid)) return e;
+        if (int e = tc_launch_cfg(tc_merge_bulk_kernel<CIN, C, PX, GRAY>, smem, MergeBulkCfg<CIN, C, PX>::ncols, ntiles, &grid)) return e;
         ProfScope ps(C == 32 ? "det_merge_c32" : "det_merge_c64", st);
-        tc_merge_bulk_kernel<CIN, C, PX><<<grid, NT2, smem, st>>>(xin, w, p, g, u, v, r, q, partial);
+        tc_merge_bulk_kernel<CIN, C, PX, GRAY><<<grid, NT2, smem, st>>>(xin, w, p, g, u, v, r, q, partial);
     } else {
         const TcPlan& p = P.merge[level];
         BALF_REQUIRE((!MergeCfg<C, PX>::bulk_uv || g.total_units % 2 == 0), "internal: odd unit count at stage %d", level);
@@ -2293,6 +2395,13 @@ int tc_run_head(const float* r, const float* q, const float* scale, const balf_d
                 const float* blob, int Bc, int hc, int wc, float* logits, float* prob, cudaStream_t st, int px, int r16) {
     return px ? tc_head_px<1>(r, q, scale, a, blob, Bc, hc, wc, logits, prob, st, r16)
               : tc_head_px<0>(r, q, scale, a, blob, Bc, hc, wc, logits, prob, st, r16);
+}
+
+int tc_run_gray_level0(const uint8_t* g, const DownW& w, const balf_detector_arch& a, const float* blob, int Bc, int h, int wd,
+                       float* u, float* v, float* r, float* q, float* partial, cudaStream_t st) {
+    TcPlans P;
+    tc_build_plans(a, blob, &P, 0);
+    return tc_run_level<3, 32, 0, true>(reinterpret_cast<const float*>(g), w, P, 0, Bc, h, wd, u, v, r, q, partial, st, 0);
 }
 #endif  // BALF_TC_MAIN
 

@@ -32,15 +32,24 @@ def _detect_device(args, im, detector, device):
     return xy[0], (dxdy[0] if dxdy is not None else None), sc[0], int(cnt[0])
 
 
+def _prob_u8(u8, detector, precision):
+    """u8 [B,H,W,C] uint8 CUDA -> (prob [B,Hp,Wp], (top, left)).  A gray image at 'tf32' takes the byte-plane forward
+    (``forward_gray``: stage 1 from per-byte tables, bit-identical to the fp32-input forward); everything else the fp32 input."""
+    with torch.inference_mode():
+        if u8.shape[3] == 1 and precision == "tf32":
+            g, (top, left) = _capi.pad_gray_u8(u8)
+            return detector.forward_gray(g, precision=precision)["prob"], (top, left)
+        x, (top, left) = _capi.preprocess_u8(u8)
+        return detector(x, precision=precision, want_logits=False)["prob"], (top, left)
+
+
 def detect_batch_device(args, u8, detector, nms="greedy"):
     """Batched device-resident detect: u8 [B,H,W,C] uint8 CUDA -> (xy int32 [B,K,2], score fp32
     [B,K], dxdy fp32 [B,K,2] | None, count int32 [B]) on the device.  ``nms`` selects the demo
     path ('greedy': demo_match.py:44-57) or the validation path ('windowed':
     balf/utils/train_utils.py:446-452)."""
     B, h, w, _ = u8.shape
-    x, (top, left) = _capi.preprocess_u8(u8)
-    with torch.inference_mode():
-        prob = detector(x, precision=detector.resolve_precision(nms), want_logits=False)["prob"]
+    prob, (top, left) = _prob_u8(u8, detector, detector.resolve_precision(nms))
     if nms == "windowed":
         xy, sc, cnt = _capi.windowed_nms_topk(prob, args.num_features, border=args.border_size,
                                               nms_size=args.nms_size, crop=(top, left, h, w))
@@ -66,11 +75,11 @@ def detect_multiscale_batch_device(args, u8, detector, scale=0.7, levels=3, nms=
     for l in range(-int(upsampled_levels), levels):
         hs, ws = _capi.level_size(h, scale, l), _capi.level_size(w, scale, l)
         if l == 0:
-            x, (top, left) = _capi.preprocess_u8(u8)
+            prob, (top, left) = _prob_u8(u8, detector, detector.resolve_precision(nms))
         else:
             x, (top, left) = _capi.resize_preprocess_u8(u8, hs, ws)
-        with torch.inference_mode():
-            prob = detector(x, precision=detector.resolve_precision(nms), want_logits=False)["prob"]
+            with torch.inference_mode():
+                prob = detector(x, precision=detector.resolve_precision(nms), want_logits=False)["prob"]
         if nms == "windowed":
             xy, sc, cnt = _capi.windowed_nms_topk(prob, args.num_features, border=args.border_size,
                                                   nms_size=args.nms_size, crop=(top, left, hs, ws))

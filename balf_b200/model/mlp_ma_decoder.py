@@ -134,3 +134,18 @@ class MLP_MA_DECODER(nn.Module):
         precision = precision or self.resolve_precision()
         logits, prob = _capi.detector_forward(x, self._weights(x.device), self.arch, precision, want_logits=want_logits)
         return {"logits": logits, "prob": prob}
+
+    def forward_gray(self, g, precision=None, want_logits=False):
+        """``forward`` for a gray uint8 image given as its padded byte plane g [B,Hp,Wp] uint8 (``_capi.pad_gray_u8``): the
+        result is bit-identical to ``forward(preprocess_u8(img)[0], 'tf32')``, but stage 1 gathers its pixel-local chain from
+        per-byte tables instead of computing it per pixel (balf_detector_forward_gray).  Only 'tf32' exists on this path;
+        ``precision=None`` means 'tf32' unless ``self.precision`` names another (which then raises)."""
+        if self.training:
+            raise RuntimeError("balf_b200 implements the inference path only: call .eval() first")
+        if not g.is_cuda:
+            raise RuntimeError("balf_b200 has no CPU path: move the model and the input to a CUDA device")
+        if self.arch["dims"][0] != 3:
+            raise ValueError("forward_gray needs a detector with a 3-channel input, this one has %d" % self.arch["dims"][0])
+        precision = precision or ("tf32" if self.precision == "auto" else self.precision)
+        logits, prob = _capi.detector_forward_gray(g, self._weights(g.device), self.arch, precision, want_logits=want_logits)
+        return {"logits": logits, "prob": prob}

@@ -73,6 +73,10 @@ BALF_API int balf_detector_pack_weights(const balf_detector_arch* arch, const fl
 BALF_API int balf_pad_geometry(int H, int W, int factor, int* Hp, int* Wp, int* top, int* left);
 BALF_API int balf_preprocess_u8(const uint8_t* img, int B, int H, int W, int C, float* x, int Hp, int Wp, int top,
                        int left, void* stream);
+/* balf_pad_gray_u8: img [B,H,W,1] uint8 (a gray image) -> g [B,Hp,Wp] uint8: the same geometry as balf_preprocess_u8 without the
+ *     conversion -- the image bytes at (top, left), zeros in the padding.  Hp and Wp must be multiples of 64.  This is the input of
+ *     balf_detector_forward_gray (1 byte per pixel instead of the 12 of the replicated fp32 planes). */
+BALF_API int balf_pad_gray_u8(const uint8_t* img, int B, int H, int W, uint8_t* g, int Hp, int Wp, int top, int left, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * D1 + D2  detector forward
@@ -89,6 +93,20 @@ BALF_API size_t balf_detector_workspace_bytes(const balf_detector_arch* arch, in
 BALF_API int balf_detector_forward(const balf_detector_arch* arch, const float* packed, const float* x, int B, int Hp,
                           int Wp, float* logits, float* prob, void* workspace, size_t workspace_bytes,
                           int precision, void* stream);
+/* balf_detector_forward_gray: balf_detector_forward for a gray uint8 image, given as its padded byte plane
+ *     g [B,Hp,Wp] uint8 (balf_pad_gray_u8) instead of x.  The result is bit-identical to balf_detector_forward on
+ *     balf_preprocess_u8 of the same image (logits and prob alike), at the same precision.
+ *   - precision must be 1; 0 and 2 are argument errors.  So is a stage-1 bit cleared by balf_debug_set(0, ...): stage 1
+ *     exists only on the tensor cores here.  An argument error launches nothing.
+ *   - Why it is faster: every pixel of the network-input stage is one of 256 byte values, and the chain of that stage up to
+ *     the token mixing (conv.0 -> ReLU -> LayerNorm -> dense1 -> GELU -> LayerNorm -> gMLP dense1 -> GELU -> LayerNorm) depends
+ *     on the pixel alone.  Each CTA of the stage-1 branch kernels tabulates it for the 256 values with the same device code,
+ *     then gathers a tile's rows from that table; the merge kernel reads 1 byte instead of 12 per pixel.  Stages 2-4, the
+ *     channel attention, the pooling and the head are those of balf_detector_forward.
+ *   - Same Hp / Wp rules, the same workspace (balf_detector_workspace_bytes) and the same outputs as balf_detector_forward. */
+BALF_API int balf_detector_forward_gray(const balf_detector_arch* arch, const float* packed, const uint8_t* g, int B, int Hp,
+                               int Wp, float* logits, float* prob, void* workspace, size_t workspace_bytes,
+                               int precision, void* stream);
 /* development hook, no reference counterpart: key 0 = bit mask of detector stages that run on the tensor-core
  * kernels when precision >= 1 (bits 0-3: the four Down stages, bit 4: the head; default all); key 1 = images per
  * internal pass of balf_detector_forward (default 16; query the workspace size again after changing it). */
